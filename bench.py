@@ -2,7 +2,8 @@
 """bench.py - depth maps / s of the A-TVSNet inference hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload cfg2|cfg3|cfg4] [--precision fp16|bf16|fp32] [--no-graph]
+                    [--workload cfg2|cfg3|cfg4] [--precision fp16|bf16|fp32] [--no-graph] [--dump-outputs DIR]
+                    [--ref-budget-s S]
 
 One "step" = one depth map of the workload: stage I (TVSNet_base_siamese: fused warp + cost volume -> 3-D CNN
 regularisation -> soft-argmin, forward and reverse direction) for every source view, stage II (attention aggregation
@@ -17,8 +18,11 @@ N > 1   : independent reference frames data-parallel, one frame stream per rank,
           sharded over the ranks, completed with an NCCL max + reduce-scatter + all-gather - and reports it under
           "sharded" (with the same frame on rank 0 alone beside it).  --workload cfg3 makes that the headline instead.
 --impl reference : the CPU oracle (NumPy/torch-CPU restatement of the TF-1.5 reference, which cannot be installed
-          offline) on all host cores; each step is the FULL workload (every depth plane, every view); the number of timed
-          steps is capped so that the run ends within a few minutes and the JSON line says how many were timed.
+          offline) on all host cores; each step is the FULL workload (every depth plane, every view, ~30 s at cfg2); all
+          --steps are timed unless --ref-budget-s S stops the run once the next step would end after S seconds (the
+          JSON line says how many were timed).
+--dump-outputs DIR : after the timed steps, rank 0 writes what the last timed step returned (the run_multiview dict)
+          as DIR/<name>.npy, so that two builds can be compared output for output on the same seeded inputs.
 """
 import argparse
 import json
@@ -39,7 +43,10 @@ WORKLOADS = {
 }
 METRIC = "depth maps/sec"
 CRM_MAC_PER_VOXEL = 29592          # SURVEY.md 8(a) a6
-REF_BUDGET_S = float(os.environ.get('ATVS_REF_BUDGET_S', '240'))
+# --dump-outputs: an array above DUMP_MAX_ELEMS elements is stored as a seeded sample of that many (8 MB as float32);
+# the five arrays of a step then stay under DUMP_MAX_BYTES even at cfg3
+DUMP_MAX_ELEMS = 1 << 21
+DUMP_MAX_BYTES = 64 << 20
 
 
 def peaks():
@@ -156,13 +163,15 @@ def run_reference(args, rank, world):
         dt = time.perf_counter() - t0
         (warm if i < nwarm else times).append(dt)
         i += 1
-        if i >= nwarm + 1 and time.perf_counter() - t_run + dt > REF_BUDGET_S:
-            break                           # bounded run: stop once the next step would cross the budget
+        if (args.ref_budget_s is not None and i >= nwarm + 1
+                and time.perf_counter() - t_run + dt > args.ref_budget_s):
+            break                           # opt-in bounded run: stop once the next step would cross the budget
     t = float(np.mean(times))
     value = 1.0 / t
+    budget = "" if args.ref_budget_s is None else " inside a %.0f s budget" % args.ref_budget_s
     sample = ("full %s workload per step (all %d depth planes, %d source views, %dx%d features), %d of %d requested steps "
-              "timed inside a %.0f s budget, %d warm-up step(s)" % (workload, D, nv - 1, H // 4, W // 4, len(times), args.steps,
-                                                                   REF_BUDGET_S, len(warm)))
+              "timed%s, %d warm-up step(s)" % (workload, D, nv - 1, H // 4, W // 4, len(times), args.steps, budget,
+                                               len(warm)))
     print(json.dumps({
         "impl": "reference", "metric": METRIC, "value": value, "unit": "depth maps/s", "n_gpus": args.gpus,
         "steps": len(times), "steps_requested": args.steps, "warmup": len(warm), "ms_per_step": 1e3 * t,
@@ -189,6 +198,32 @@ def capture(step_fn, torch):
         graph.replay()
     torch.cuda.synchronize()
     return graph, out
+
+
+def dump_outputs(out, directory):
+    """write one step's result (the run_multiview dict) as directory/<name>.npy, float32 (float64 stays float64);
+    depth_views is stacked along a new leading axis.  An array of more than DUMP_MAX_ELEMS elements is replaced by
+    that many of its flattened elements at sorted indices drawn with a fixed seed: the same indices in every run."""
+    import numpy as np
+    import torch
+    arrays = {}
+    for name, t in out.items():
+        if isinstance(t, list):
+            if any(x is None for x in t):
+                continue                    # depth_views of a step without the reverse passes
+            t = torch.stack(t)
+        t = t.detach()
+        if t.numel() > DUMP_MAX_ELEMS:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), DUMP_MAX_ELEMS, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        t = t.double() if t.dtype == torch.float64 else t.float()
+        arrays[name] = t.cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError("bench: %d bytes of outputs exceed the %d-byte dump limit" % (total, DUMP_MAX_BYTES))
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + '.npy'), a)
 
 
 def timed_steps(fn, steps, torch, barrier):
@@ -237,7 +272,7 @@ def run_ours(args, rank, world, local_rank):
 
     def step():
         return A.pipeline.run_multiview(feats_d, cams_d, D, siamese=True, upsample=True, group=group, rank=rank,
-                                        world=world)['depth_up']
+                                        world=world)
 
     def barrier():
         if world > 1:
@@ -272,6 +307,12 @@ def run_ours(args, rank, world, local_rank):
     sampler.wait_first()
     barrier()
     ms_total, res = timed_steps(run_step, args.steps, torch, barrier)
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        # a device copy now (the graph and its buffers are released below); the files are written once the clock
+        # sampler has stopped, so that the host work of the dump does not enter the clocks of the timed regions
+        dumped = {k: [x if x is None else x.clone() for x in v] if isinstance(v, list) else v.clone()
+                  for k, v in res.items()}
 
     # ---------------- timed region 2: end to end from / to pinned host memory ----------------
     # the public streaming call (pipeline.FrameStream): frames arrive in pinned host memory, every step copies its
@@ -297,10 +338,13 @@ def run_ours(args, rank, world, local_rank):
             feats_d.copy_(feats_h, non_blocking=True)
             cams_d.copy_(cams_h, non_blocking=True)
             res = run_step()
-            depth_h.copy_(res, non_blocking=True)
+            depth_h.copy_(res['depth_up'], non_blocking=True)
     f1.record()
     barrier()
     clocks = sampler.stop()
+    if dumped is not None:
+        dump_outputs(dumped, args.dump_outputs)
+        dumped = None
     ms_e2e = f0.elapsed_time(f1)
     # sanity of what was timed: the depth map must be finite and inside the swept inverse-depth range
     dmin, dmax = float(cams[0, 0, 1, 3, 0]), float(cams[0, 0, 1, 3, 0] + (D - 1) * cams[0, 0, 1, 3, 1])
@@ -739,7 +783,15 @@ def main():
     ap.add_argument('--no-extras', action='store_true',
                     help='skip the extra fields (from-images / four-stage at N=1, sharded cfg3 at N>1)')
     ap.add_argument('--no-cpu-baseline', action='store_true')
+    ap.add_argument('--ref-budget-s', type=float, default=None, metavar='S',
+                    help='--impl reference: time fewer than --steps steps if the run would otherwise pass S seconds')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed step returned as DIR/<name>.npy (rank 0)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the outputs of --impl ours only')
 
     rank = int(os.environ.get('RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))

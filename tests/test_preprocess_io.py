@@ -40,24 +40,22 @@ def test_load_cam_depth_field_variants():
 
 
 def test_write_cam_round_trip(tmp_path):
-    ref = '/root/reference/example/0/2_cam.npy'
-    if os.path.exists(ref):
-        cam = np.load(ref).astype(np.float64)
-    else:
-        rng = np.random.default_rng(0)
-        cam = np.zeros((2, 4, 4))
-        cam[0] = np.eye(4)
-        cam[0, :3] = rng.standard_normal((3, 4))
-        cam[1, :3, :3] = [[131.7, 0, 120], [0, 132.1, 80], [0, 0, 1]]
-        cam[1, 3] = [0.05, 0.0033, 128, 0.4724]
-    f = str(tmp_path / 'c_cam.txt')
-    P.write_cam(f, cam)
-    back = P.load_cam(f)
-    assert np.array_equal(back[0], cam[0]) and np.array_equal(back[1, :3, :3], cam[1, :3, :3])
-    assert np.array_equal(back[1, 3], cam[1, 3])
-    s = P.scale_camera(cam, 0.25)
-    assert s[1, 0, 0] == cam[1, 0, 0] * 0.25 and s[1, 1, 2] == cam[1, 1, 2] * 0.25 and s[1, 2, 2] == cam[1, 2, 2]
-    assert np.array_equal(s[0], cam[0]) and s is not cam
+    bundled = np.load(os.path.join(ROOT, 'tests', 'golden', 'example', '0', '2_cam.npy')).astype(np.float64)
+    rng = np.random.default_rng(0)
+    posed = np.zeros((2, 4, 4))         # random pose, all four depth fields set
+    posed[0] = np.eye(4)
+    posed[0, :3] = rng.standard_normal((3, 4))
+    posed[1, :3, :3] = [[131.7, 0, 120], [0, 132.1, 80], [0, 0, 1]]
+    posed[1, 3] = [0.05, 0.0033, 128, 0.4724]
+    for cam in (bundled, posed):
+        f = str(tmp_path / 'c_cam.txt')
+        P.write_cam(f, cam)
+        back = P.load_cam(f)
+        assert np.array_equal(back[0], cam[0]) and np.array_equal(back[1, :3, :3], cam[1, :3, :3])
+        assert np.array_equal(back[1, 3], cam[1, 3])
+        s = P.scale_camera(cam, 0.25)
+        assert s[1, 0, 0] == cam[1, 0, 0] * 0.25 and s[1, 1, 2] == cam[1, 1, 2] * 0.25 and s[1, 2, 2] == cam[1, 2, 2]
+        assert np.array_equal(s[0], cam[0]) and s is not cam
 
 
 def test_pfm_round_trip_and_layout(tmp_path):
