@@ -6,8 +6,7 @@ import os
 import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# ATVS_LIB: alternative build of the same library (e.g. the -DATVS_RING_TRACE instrumented one)
-_SO = os.environ.get("ATVS_LIB") or os.path.join(_HERE, "libatvs.so")
+_SO = os.path.join(_HERE, "libatvs.so")
 _lib = None
 
 F32, BF16, F16 = 0, 1, 2

@@ -22,7 +22,6 @@
 #include "ring_common.cuh"
 #include "conv_ring.cuh"
 #include <cstring>
-#include <cstdlib>
 
 namespace {
 
@@ -55,10 +54,10 @@ struct AUnit {
 
 struct AUnitIter {
     RingSpan span;
-    __device__ __forceinline__ explicit AUnitIter(const AttnParams& p) : span(1, p.total, 0) {}
+    __device__ __forceinline__ explicit AUnitIter(const AttnParams& p) : span(p.total) {}
     __device__ __forceinline__ bool next(const AttnParams& p, AUnit& r) {
         long long t;
-        if (!span.next(1, p.D, 0, 0, t, r.z0, r.zlen)) return false;
+        if (!span.next(p.D, t, r.z0, r.zlen)) return false;
         r.x0 = (int)(t % p.nXT) * AR_TX;
         t /= p.nXT;
         r.y0 = (int)(t % p.nYT) * AR_TY;
@@ -392,7 +391,6 @@ int launch_attn(const AttnParams& p, const uint8_t* wimg, float* out, size_t sme
 }  // namespace
 
 bool attn_ring_applicable(int n_views, int D, int H, int W) {
-    if (const char* e = getenv("ATVS_ATTN_FUSED")) if (atoi(e) == 0) return false;
     return n_views >= 2 && n_views <= AR_MAXV && D >= 3 && H >= 8 && W >= 8;
 }
 
@@ -416,24 +414,16 @@ int attn_ring(const void* const* views, int n_views, int dtype, const void* wimg
     const size_t fixed = 128 + (size_t)((p.wbytes + 127) & ~127) + (2 * AR_MAXR + 2 * AR_MAXG + 1) * 8 + 16;
     const size_t budget = (minb == 2 ? 110 : 220) * 1024;
     int nring = (int)((budget - fixed) / slot);
-    {
-        int cap = 8;
-        if (const char* e = getenv("ATVS_ATTN_R")) cap = atoi(e) >= 2 && atoi(e) <= AR_MAXR ? atoi(e) : cap;
-        if (nring > cap) nring = cap;
-    }
+    if (nring > 8) nring = 8;
     if (nring < 2) {
         atvs_set_error("atvs_attention_fused: ring does not fit");
         return ATVS_E_UNSUP;
     }
     p.nring = nring;
     p.pf = nring - 1 < 4 ? nring - 1 : 4;
-    if (const char* e = getenv("ATVS_ATTN_PF")) {
-        const int v = atoi(e);
-        if (v >= 1 && v < nring && v <= 4) p.pf = v;
-    }
     const size_t smem = fixed + (size_t)nring * slot;
     const int sms = atvs_num_sms();
-    const int grid = ring_balanced_grid(p.total, (long long)sms * minb, 12, 40, "ATVS_ATTN_CTAS", nullptr);
+    const int grid = ring_balanced_grid(p.total, (long long)sms * minb, 12, 40);
     const uint8_t* wi = (const uint8_t*)wimg;
 #define AT_CASE(NM, GG, MB)                                                                                  \
     return p.f16 ? launch_attn<NM, GG, MB, true>(p, wi, out, smem, grid, st)                                 \

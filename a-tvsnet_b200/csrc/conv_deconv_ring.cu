@@ -18,13 +18,12 @@
 //               whose kz=2 taps complete output plane 2*z0)
 //   warps 0-3 producers (cp.async, zero fill = outside the volume) | warp 4 MMA issuer | warps 5-12 epilogue:
 //   two sets of four warps (one per TMEM lane quarter), set 0 drains the even output planes, set 1 the odd ones -
-//   the per-role timelines (tools/build_trace.sh, profiles/r02_deconv_ring_trace.txt) showed ONE set as the critical
+//   the per-role timelines (profiles/r02_deconv_ring_trace.txt) showed ONE set as the critical
 //   path at ~1600 cycles per input plane (convert + store + moments of 2 x 128 x 32 values on 4 warps) with the MMA
 //   warp waiting for accumulators.  Accumulation is always "+=": the epilogue zeroes a group right after reading it.
 #include "ring_common.cuh"
 #include "conv_deconv.cuh"
 #include <cstring>
-#include <cstdlib>
 
 namespace {
 
@@ -42,12 +41,10 @@ struct DrParams {
     int raw16;              // raw output dtype: 0 fp32, 1 saturated fp16
     uint32_t fmt;           // operand format bits of the instruction descriptor (tc_fmt_bits)
     unsigned long long* sat;   // saturation counter of the fp16 raw stores (atvs_sat_ptr)
-    int nXT, nYT, nZS, ZS;
+    int nXT, nYT;
     int nring, pf;
     int wbytes;
-    long long nunits;
-    int balanced;           // ring_common.cuh RingSpan: 1 = balanced ranges of input planes
-    long long total;        // tile columns * D
+    long long total;        // tile columns * D: the input plane sequence cut into one range per CTA (RingSpan)
 };
 
 template <int CIN, int COUT>
@@ -69,10 +66,10 @@ struct DrUnit {
 
 struct DrIter {
     RingSpan span;
-    __device__ __forceinline__ explicit DrIter(const DrParams& p) : span(p.balanced, p.total, p.nunits) {}
+    __device__ __forceinline__ explicit DrIter(const DrParams& p) : span(p.total) {}
     __device__ __forceinline__ bool next(const DrParams& p, DrUnit& r) {
         long long t;
-        if (!span.next(p.balanced, p.D, p.nZS, p.ZS, t, r.z0, r.zlen)) return false;
+        if (!span.next(p.D, t, r.z0, r.zlen)) return false;
         r.x0 = (int)(t % p.nXT) * DR_TX;
         t /= p.nXT;
         r.y0 = (int)(t % p.nYT) * DR_TY;
@@ -173,7 +170,6 @@ k_deconv3d_ring(const uint16_t* __restrict__ x, const __grid_constant__ DrParams
             }
         };
         const size_t zstride_in = (size_t)p.H * p.W * CIN;
-        TRACE_DECL
         DrIter units(p);
         DrUnit un;
         while (units.next(p, un)) {
@@ -191,7 +187,6 @@ k_deconv3d_ring(const uint16_t* __restrict__ x, const __grid_constant__ DrParams
             const uint16_t* zbase = x + ((size_t)un.b * p.D + (un.z0 + ibeg)) * zstride_in;
             for (int i = ibeg; i < un.zlen; ++i, zbase += zstride_in) {
                 mbar_wait(&empty[slot], sphase ^ 1);
-                TRACE(0);
                 const uint32_t dst0 = ring_u32 + slot * (uint32_t)Cfg::SLOT_BYTES;
 #pragma unroll
                 for (int k = 0; k < NITEM; ++k) {
@@ -206,15 +201,11 @@ k_deconv3d_ring(const uint16_t* __restrict__ x, const __grid_constant__ DrParams
                     }
                 }
                 asm volatile("cp.async.commit_group;" ::: "memory");
-                TRACE(1);
                 if (++slot == (uint32_t)R) { slot = 0; sphase ^= 1; }
                 if (++pending >= (uint32_t)PF) publish(PF - 1);
-                TRACE(2);
-                TRACE_NEXT();
             }
         }
         publish(0);
-        if (ptid == 0) TRACE_DUMP("P");
     } else if (warp == 4) {
         // ===================== MMA issuer (one elected thread) =====================
         if (elect_one()) {
@@ -237,7 +228,6 @@ k_deconv3d_ring(const uint16_t* __restrict__ x, const __grid_constant__ DrParams
             };
             uint32_t slot = 0, sphase = 0;
             uint32_t gq = 0, gphase = 0;       // accumulator group / phase of output plane t = 0 of the unit
-            TRACE_DECL
             DrIter units(p);
             DrUnit un;
             while (units.next(p, un)) {
@@ -256,9 +246,7 @@ k_deconv3d_ring(const uint16_t* __restrict__ x, const __grid_constant__ DrParams
                         ++twaited;
                         if (++gw == (uint32_t)G) { gw = 0; gwphase ^= 1; }
                     }
-                    TRACE(0);
                     mbar_wait(&full[slot], sphase);
-                    TRACE(1);
                     tc_fence_after();
                     const uint32_t a_lo0 = a_lo_ring + slot * (uint32_t)(Cfg::SLOT_BYTES >> 4);
                     uint32_t glo = gq + (uint32_t)tlo;
@@ -279,12 +267,9 @@ k_deconv3d_ring(const uint16_t* __restrict__ x, const __grid_constant__ DrParams
                         tc_commit(&tfull[gdone]);
                         if (++gdone == (uint32_t)G) gdone = 0;
                     }
-                    TRACE(2);
-                    TRACE_NEXT();
                 }
                 gq = gw; gphase = gwphase;
             }
-            TRACE_DUMP("M");
         }
         __syncwarp();
     } else {
@@ -302,7 +287,6 @@ k_deconv3d_ring(const uint16_t* __restrict__ x, const __grid_constant__ DrParams
         const int Ho = 2 * p.H, Wo = 2 * p.W, Do = 2 * p.D;
         // a unit starts on an even group and consumes an even number of groups: set s only ever sees groups of parity s
         uint32_t grp = (uint32_t)set, gphase = 0;
-        TRACE_DECL
         DrIter units(p);
         DrUnit un;
         while (units.next(p, un)) {
@@ -311,7 +295,6 @@ k_deconv3d_ring(const uint16_t* __restrict__ x, const __grid_constant__ DrParams
             const int nt = 2 * un.zlen;
             for (int t = set; t < nt; t += 2) {
                 mbar_wait(&tfull[grp], gphase);
-                TRACE(0);
                 tc_fence_after();
                 const uint32_t taddr = tmem_base + ((uint32_t)(g * 32) << 16) + grp * (uint32_t)GC;
                 uint64_t* const tempty_bar = &tempty[grp];
@@ -327,8 +310,7 @@ k_deconv3d_ring(const uint16_t* __restrict__ x, const __grid_constant__ DrParams
                 tc_fence_before();
                 __syncwarp();
                 if (lane == 0) mbar_arrive(tempty_bar);
-                TRACE(1);
-                if (!ok) { TRACE_NEXT(); continue; }
+                if (!ok) continue;
                 const int oz = 2 * un.z0 + t;
 #pragma unroll
                 for (int py = 0; py < 2; ++py) {
@@ -348,13 +330,10 @@ k_deconv3d_ring(const uint16_t* __restrict__ x, const __grid_constant__ DrParams
                         run[COUT + c % COUT] = fmaf(r, r, run[COUT + c % COUT]);
                     }
                 }
-                TRACE(2);
-                TRACE_NEXT();
             }
         }
         // fp16 raw output: count the threads that had to clamp a value (atvs_saturation_count)
         if (p.raw16 && p.sat != nullptr && vmax > 65504.f) atomicAdd(p.sat, 1ULL);
-        if (warp == 5 && lane == 0) TRACE_DUMP("E");
         if (stats != nullptr) {
 #pragma unroll
             for (int k = 0; k < 2 * COUT; ++k) {
@@ -415,12 +394,10 @@ size_t dr_wbytes(int Cin, int Cout) { return (size_t)4 * (Cin / 16) * 2 * (3 * 4
 bool deconv_ring_supported(int Cin, int Cout) { return (Cin == 16 && Cout == 8) || (Cin == 32 && Cout == 16); }
 
 bool deconv_ring_applicable(int B, int D, int H, int W) {
-    if (getenv("ATVS_NO_DECONV_RING") != nullptr) return false;
     // alone, the per-(class, tap) kernel is faster below ~100k input voxels (18.6 vs 30 us for 32 -> 16 on 32x32x40), but
     // inside the step the plane ring wins there too (5.93 vs 6.08 ms per cfg2 depth map: 110 KB of shared memory and 8
     // staged TMA tiles per 128 voxels less pressure on the co-running passes)
-    const long long minvox = getenv("ATVS_DECONV_RING_MINVOX") ? atoll(getenv("ATVS_DECONV_RING_MINVOX")) : 16384;
-    return (long long)B * D * H * W >= minvox && H >= 2 && W >= 2;
+    return (long long)B * D * H * W >= 16384 && H >= 2 && W >= 2;
 }
 
 size_t deconv_ring_weight_bytes(int Cin, int Cout) {
@@ -453,7 +430,6 @@ int deconv_ring(const void* x16, int dtype, const void* wimg, int B, int D, int 
     const size_t budget = 110 * 1024;
     int nring = (int)((budget - fixed) / slot);
     if (nring > 12) nring = 12;
-    if (const char* e = getenv("ATVS_DRING_R")) nring = atoi(e) >= 2 && atoi(e) < nring ? atoi(e) : nring;
     if (nring < 2) {
         atvs_set_error("atvs_conv3d_tc(deconv ring): weights do not fit next to 2 ring planes (Cin=%d Cout=%d)", Cin, Cout);
         return ATVS_E_UNSUP;
@@ -462,24 +438,9 @@ int deconv_ring(const void* x16, int dtype, const void* wimg, int B, int D, int 
     // planes of cp.async in flight per producer thread (the loads queue behind the kernel's own 8x larger write stream:
     // ~4000 cycles of latency in the timelines), at most nring - 1 and 8
     p.pf = nring - 1 < 8 ? nring - 1 : 8;
-    if (const char* e = getenv("ATVS_DRING_PF")) p.pf = atoi(e) >= 1 && atoi(e) < p.pf ? atoi(e) : p.pf;
-    {   // input z segment length: minimise waves * (planes per unit)
-        const long long cols = (long long)B * p.nXT * p.nYT;
-        const long long slots = (long long)sms * minb;
-        int bz = ring_pick_zs(cols, D, slots, 1, 1, 0.4, 10.0, 2);
-        if (const char* e = getenv("ATVS_DRING_ZS")) bz = atoi(e) > 0 && atoi(e) <= D ? atoi(e) : bz;
-        p.ZS = bz;
-        p.nZS = (D + bz - 1) / bz;
-        p.nunits = cols * p.nZS;
-    }
+    p.total = (long long)B * p.nXT * p.nYT * D;
     const size_t smem = fixed + (size_t)nring * slot;
-    int grid = (int)(p.nunits < (long long)sms * minb ? p.nunits : (long long)sms * minb);
-    {   // balanced ranges of input planes (default, ring_common.cuh); ATVS_DRING_BALANCED=0: fixed z segments
-        p.total = (long long)B * p.nXT * p.nYT * D;
-        p.balanced = 1;
-        if (const char* e = getenv("ATVS_DRING_BALANCED")) p.balanced = atoi(e) != 0;
-        if (p.balanced) grid = ring_balanced_grid(p.total, (long long)sms * minb, 20, 160, "ATVS_DRING_CTAS", nullptr);
-    }
+    const int grid = ring_balanced_grid(p.total, (long long)sms * minb, 20, 160);
     const uint8_t* wi = (const uint8_t*)wimg;
     if (Cin == 16 && Cout == 8) return launch_dr<16, 8>((const uint16_t*)x16, p, wi, raw_out, stats, smem, grid, st);
     if (Cin == 32 && Cout == 16) return launch_dr<32, 16>((const uint16_t*)x16, p, wi, raw_out, stats, smem, grid, st);

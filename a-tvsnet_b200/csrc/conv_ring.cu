@@ -36,29 +36,22 @@
 #include "ring_common.cuh"
 #include "conv_ring.cuh"
 #include <cstring>
-#include <cstdlib>
 
 namespace {
 
 
-// one CTA plane = MT MMA tiles (16 y x 8 x each) side by side in x: MT = 2 (256 voxels per plane step) by default.
-// The skeleton of the three roles (no loads / MMAs / stores) runs at ~760 cycles per 256-voxel plane
-// (profiles/r02_ring_8_8_trace.txt), which is what bounds the 8-channel layers; MT = 4 (512 voxels, 7-group accumulator
-// ring so that two CTAs still share the 512 TMEM columns) and grouped publishing of planes (PG) were built to amortise
-// it and measured: neither changes the 45 us of an 8 -> 8 layer at cfg2 (profiles/r02_ring_probe.txt), so the cost
-// scales with the plane, not with the handshake count.
+// one CTA plane = RG_MT = 2 MMA tiles (16 y x 8 x each) side by side in x: 256 voxels per plane step, published as one
+// cp.async group.  The skeleton of the three roles (no loads / MMAs / stores) runs at ~760 cycles per 256-voxel plane
+// (profiles/r02_ring_8_8_trace.txt), which is what bounds the 8-channel layers; 4-tile planes (512 voxels, 7-group
+// accumulator ring so that two CTAs still share the 512 TMEM columns) and grouped publishing of 2-4 planes were built to
+// amortise it and measured: neither changes the 45 us of an 8 -> 8 layer at cfg2 (profiles/r02_ring_probe.txt), so the
+// cost scales with the plane, not with the handshake count.
 constexpr int RG_TY = 16, RG_HH = RG_TY + 2;
+constexpr int RG_MT = 2, RG_TX = 8 * RG_MT, RG_WW = RG_TX + 2;
 constexpr int RG_PRODUCERS = 128;
 constexpr int RG_THREADS = 288;
 constexpr int RG_MAXG = 15;
-constexpr int RG_MAXR = 16;      // ring slots (mbarrier pairs)
-#ifndef RING_NOINC_DEFAULT
-#define RING_NOINC_DEFAULT 0
-#endif
-#ifndef RING_LATE_RELEASE
-#define RING_LATE_RELEASE 0       // 1: release an accumulator group after the plane's stores instead of before them (zeroing
-                                  // overlapped with the conversion): measured 31.7 vs 31.9 us per 8 -> 8 layer in steady state, kept off
-#endif
+constexpr int RG_MAXR = 16;      // mbarrier pairs reserved for the ring slots
 
 struct RingParams {
     int B, D, H, W;
@@ -66,31 +59,26 @@ struct RingParams {
     int raw16;          // raw output dtype: 0 fp32, 1 saturated fp16
     uint32_t fmt;       // operand format bits of the instruction descriptor (tc_fmt_bits)
     unsigned long long* sat;   // saturation counter of the fp16 raw stores (atvs_sat_ptr)
-    int nXT, nYT, nZS, ZS, TX;   // TX = tile width in voxels (8 * MT)
-    int nring, pf, pg;  // ring slots; cp.async GROUPS in flight per producer thread; planes per group (pf * pg < nring)
+    int nXT, nYT;
+    int nring, pf;      // ring slots; planes of cp.async in flight per producer thread (pf < nring)
     int wbytes;
-    int dbg;            // ATVS_RING_DEBUG bit mask (tools/conv_probe.py): 1 no loads, 2 no MMAs, 4 no stores, 8 no zeroing
-    long long nunits;
-    int noinc;          // 1: planes published by cp.async.mbarrier.arrive.noinc (producers never wait), consumer-side proxy fence
-    int balanced;       // 1: every CTA owns one contiguous range of the linear (tile column, z) plane sequence
-    long long total;    // balanced: tile columns * D
+    long long total;    // tile columns * D: the plane sequence cut into one range per CTA (RingSpan)
 };
 
-template <int CIN, int CP, int MT>
+template <int CIN, int CP>
 struct RingCfg {
-    static constexpr int TX = 8 * MT, WW = TX + 2;
-    static constexpr int NVOX = RG_HH * WW;               // voxels of one halo plane (324 for MT = 2)
+    static constexpr int NVOX = RG_HH * RG_WW;            // voxels of one halo plane (324)
     static constexpr int KCH_PAD = NVOX * 16 + 16;        // pitch of one 8-channel chunk plane; +16 B keeps the
                                                           // 8 chunk stores of a voxel on distinct banks
     static constexpr int NKC = CIN / 8;
     static constexpr int SLOT_BYTES = (NKC * KCH_PAD + 127) / 128 * 128;
     static constexpr int NSTEPS = (CIN >= 16) ? 9 * (CIN / 16) : 5;     // K=16 MMA steps per input plane
     static constexpr bool PAD = (CP == 8);                              // runs are padded to N % 16 == 0 with zero weights
-    static constexpr int G = (CP == 8) ? (MT == 4 ? 7 : 15) : 8;        // accumulator groups in the ring
+    static constexpr int G = (CP == 8) ? 15 : 8;                        // accumulator groups in the ring
     static constexpr int NROWS = (CP == 8) ? 64 : 3 * CP;               // rows of one weight step image
     static constexpr int STEP_BYTES = 2 * NROWS * 16;
-    static constexpr uint32_t TILE_COLS = (CP == 32) ? 256u : ((CP == 8 && MT == 4) ? 64u : 128u);   // CP=8: G groups + 1 dummy
-    static constexpr uint32_t TMEM_COLS = MT * TILE_COLS;
+    static constexpr uint32_t TILE_COLS = (CP == 32) ? 256u : 128u;    // CP=8: G groups + 1 dummy
+    static constexpr uint32_t TMEM_COLS = RG_MT * TILE_COLS;
 };
 
 struct Unit {
@@ -98,14 +86,14 @@ struct Unit {
 };
 
 
-// units of this CTA (ring_common.cuh RingSpan: balanced plane ranges by default, fixed z segments on request)
+// units of this CTA (ring_common.cuh RingSpan: one balanced range of the plane sequence)
 struct UnitIter {
     RingSpan span;
-    __device__ __forceinline__ explicit UnitIter(const RingParams& p) : span(p.balanced, p.total, p.nunits) {}
+    __device__ __forceinline__ explicit UnitIter(const RingParams& p) : span(p.total) {}
     __device__ __forceinline__ bool next(const RingParams& p, Unit& r) {
         long long t;
-        if (!span.next(p.balanced, p.D, p.nZS, p.ZS, t, r.z0, r.zlen)) return false;
-        r.x0 = (int)(t % p.nXT) * p.TX;
+        if (!span.next(p.D, t, r.z0, r.zlen)) return false;
+        r.x0 = (int)(t % p.nXT) * RG_TX;
         t /= p.nXT;
         r.y0 = (int)(t % p.nYT) * RG_TY;
         r.b = (int)(t / p.nYT);
@@ -138,14 +126,14 @@ __device__ __forceinline__ void ring_window(int f, int len, uint32_t& row_off_by
     }
 }
 
-template <int CIN, int CP, int MT, int MINB, bool FAST>
+template <int CIN, int CP, int MINB, bool FAST>
 __global__ void __launch_bounds__(RG_THREADS, MINB)
 k_conv3d_ring(const uint16_t* __restrict__ x, const __grid_constant__ RingParams p,
               const uint8_t* __restrict__ wimg, float* __restrict__ out, double* __restrict__ stats,
               const float* __restrict__ bias) {
-    using Cfg = RingCfg<CIN, CP, MT>;
+    using Cfg = RingCfg<CIN, CP>;
     constexpr int G = Cfg::G;
-    constexpr int RG_WW = Cfg::WW, RG_NVOX = Cfg::NVOX, RG_KCH_PAD = Cfg::KCH_PAD, RG_MT = MT;
+    constexpr int RG_NVOX = Cfg::NVOX, RG_KCH_PAD = Cfg::KCH_PAD;
 
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>(((uintptr_t)smem_raw + 127) & ~(uintptr_t)127);
@@ -163,7 +151,7 @@ k_conv3d_ring(const uint16_t* __restrict__ x, const __grid_constant__ RingParams
     const int R = p.nring;
     if (threadIdx.x == 0) {
         for (int s = 0; s < R; ++s) {
-            mbar_init(&full[s], p.noinc ? RG_PRODUCERS : RG_PRODUCERS / 32);      // per thread (noinc) | per producer WARP
+            mbar_init(&full[s], RG_PRODUCERS / 32);      // one arrival per producer WARP (lane 0, after __syncwarp)
             mbar_init(&empty[s], 1);
         }
         for (int g = 0; g < G; ++g) {
@@ -208,17 +196,13 @@ k_conv3d_ring(const uint16_t* __restrict__ x, const __grid_constant__ RingParams
         // mbarrier arrive) once plane q+PF-1 has been issued.  PF <= R-1 keeps the ring deadlock-free.
         // Publishing a plane (cp.async.wait_group + fence.proxy.async + __syncwarp + mbarrier arrive) costs ~400 cycles of
         // the producer's per-plane loop whatever the plane holds (profiles/r02_ring_8_8_trace.txt: 770 cycles per plane
-        // with nothing to load): planes are committed and published in groups of PG, up to PF groups in flight.
-        const int PF = p.pf, PG = p.pg;
-        uint32_t slot = 0, sphase = 0, pslot = 0, pending = 0, pplanes = 0, gopen = 0;
+        // with nothing to load).
+        const int PF = p.pf;      // 1..4
+        uint32_t slot = 0, sphase = 0, pslot = 0, pending = 0;
         const uint32_t ring_u32 = smem_u32(ring);
         auto publish = [&](int keep) {
-            // wait until at most `keep` groups are pending, then publish every older plane
-            if (keep >= 7) asm volatile("cp.async.wait_group 7;" ::: "memory");
-            else if (keep == 6) asm volatile("cp.async.wait_group 6;" ::: "memory");
-            else if (keep == 5) asm volatile("cp.async.wait_group 5;" ::: "memory");
-            else if (keep == 4) asm volatile("cp.async.wait_group 4;" ::: "memory");
-            else if (keep == 3) asm volatile("cp.async.wait_group 3;" ::: "memory");
+            // wait until at most `keep` planes are pending, then publish every older plane
+            if (keep >= 3) asm volatile("cp.async.wait_group 3;" ::: "memory");
             else if (keep == 2) asm volatile("cp.async.wait_group 2;" ::: "memory");
             else if (keep == 1) asm volatile("cp.async.wait_group 1;" ::: "memory");
             else asm volatile("cp.async.wait_group 0;" ::: "memory");
@@ -226,15 +210,12 @@ k_conv3d_ring(const uint16_t* __restrict__ x, const __grid_constant__ RingParams
             // every lane's copies have landed and are visible to the async proxy; one release-arrive per warp
             // (128 per-thread arrivals on one mbarrier cost more than the plane's cp.async issue)
             __syncwarp();
-            // the groups that stay pending are full ones (a partial group only exists at the very end, flushed with keep 0)
-            for (; pplanes > (uint32_t)(keep * PG); --pplanes) {
+            for (; pending > (uint32_t)keep; --pending) {
                 if ((threadIdx.x & 31) == 0) mbar_arrive(&full[pslot]);
                 if (++pslot == (uint32_t)R) pslot = 0;
             }
-            if (pending > (uint32_t)keep) pending = (uint32_t)keep;
         };
         const size_t zstride_in = (size_t)p.H * p.W * CIN;
-        TRACE_DECL
         UnitIter units(p);
         Unit un;
         while (units.next(p, un)) {
@@ -252,11 +233,10 @@ k_conv3d_ring(const uint16_t* __restrict__ x, const __grid_constant__ RingParams
             const uint16_t* zbase = x + ((size_t)un.b * p.D + (un.z0 - 1 + ibeg)) * zstride_in;
             for (int i = ibeg; i <= iend; ++i, zbase += zstride_in) {
                 mbar_wait(&empty[slot], sphase ^ 1);
-                TRACE(0);
                 const uint32_t dst0 = ring_u32 + slot * (uint32_t)Cfg::SLOT_BYTES;
 #pragma unroll
                 for (int k = 0; k < NITEM; ++k) {
-                    if (goff[k] != -2 && !(p.dbg & 1)) {
+                    if (goff[k] != -2) {
                         const int j = ptid + k * RG_PRODUCERS;
                         const uint32_t soff = (uint32_t)((j % Cfg::NKC) * RG_KCH_PAD + (j / Cfg::NKC) * 16);
                         const bool ok = goff[k] >= 0;
@@ -266,35 +246,12 @@ k_conv3d_ring(const uint16_t* __restrict__ x, const __grid_constant__ RingParams
                                      : "memory");
                     }
                 }
-                TRACE(1);
-                if (p.noinc) {
-                    // the plane's mbarrier tracks this thread's copies: it completes when all 128 threads' copies have landed;
-                    // nothing to wait for here (the ring's `empty` barriers bound the planes in flight)
-                    asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" ::"r"(smem_u32(&full[slot])) : "memory");
-                    if (++slot == (uint32_t)R) { slot = 0; sphase ^= 1; }
-                    TRACE(2);
-                    TRACE_NEXT();
-                    continue;
-                }
                 if (++slot == (uint32_t)R) { slot = 0; sphase ^= 1; }
-                if (++gopen == (uint32_t)PG) {
-                    asm volatile("cp.async.commit_group;" ::: "memory");
-                    gopen = 0;
-                    pplanes += (uint32_t)PG;
-                    if (++pending >= (uint32_t)PF) publish(PF - 1);
-                }
-                TRACE(2);
-                TRACE_NEXT();
+                asm volatile("cp.async.commit_group;" ::: "memory");
+                if (++pending >= (uint32_t)PF) publish(PF - 1);
             }
         }
-        if (gopen > 0) {
-            asm volatile("cp.async.commit_group;" ::: "memory");
-            pplanes += gopen;
-            ++pending;
-        }
-        if (p.noinc) asm volatile("cp.async.wait_all;" ::: "memory");      // no copy outlives the CTA's shared memory
-        else publish(0);
-        if (ptid == 0) TRACE_DUMP("P");
+        publish(0);
     } else if (warp == 4) {
         // ===================== MMA issuer (elected lane) =====================
         // The instruction stream per plane matters for the small-channel layers: counters are incremental (no
@@ -331,7 +288,6 @@ k_conv3d_ring(const uint16_t* __restrict__ x, const __grid_constant__ RingParams
                                  b_lo + ((uint32_t)(s * Cfg::STEP_BYTES) >> 4), B_HI, idesc);
             }
         };
-        TRACE_DECL
         uint32_t slot = 0, sphase = 0;     // ring position of the next input plane
         uint32_t gq = 0, gphase = 0;       // accumulator group / phase of output plane t = 0 of the unit
         UnitIter units(p);
@@ -353,15 +309,10 @@ k_conv3d_ring(const uint16_t* __restrict__ x, const __grid_constant__ RingParams
                     ++twaited;
                     if (++gw == (uint32_t)G) { gw = 0; gwphase ^= 1; }
                 }
-                TRACE(0);
                 mbar_wait(&full[slot], sphase);
-                TRACE(1);
-                // cp.async wrote the plane through the generic proxy; the MMA reads it through the async proxy
-                if (p.noinc) asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
                 tc_fence_after();
                 const uint32_t a_lo0 = a_lo_ring + slot * (uint32_t)(Cfg::SLOT_BYTES >> 4);
-                if (p.dbg & 2) {
-                } else if (thi - tlo == 2 && glo + 3 <= (uint32_t)G) {
+                if (thi - tlo == 2 && glo + 3 <= (uint32_t)G) {
                     issue_plane(tmem_base + glo * (uint32_t)CP, a_lo0, b_lo0 + (FAST_BOFF >> 4), FAST_IDESC);
                 } else {
                     const int len = thi - tlo + 1, f = i - tlo;
@@ -384,8 +335,6 @@ k_conv3d_ring(const uint16_t* __restrict__ x, const __grid_constant__ RingParams
                     ++tdone;
                     if (++gdone == (uint32_t)G) gdone = 0;
                 }
-                TRACE(2);
-                TRACE_NEXT();
             }
             gq = gw; gphase = gwphase;
             if (twaited >= un.zlen) {      // the CP = 8 look-ahead waited for the next unit's first plane
@@ -393,7 +342,6 @@ k_conv3d_ring(const uint16_t* __restrict__ x, const __grid_constant__ RingParams
                 if (gq == (uint32_t)G - 1) gphase ^= 1;
             }
         }
-        TRACE_DUMP("M");
         }
         __syncwarp();
     } else {
@@ -412,8 +360,6 @@ k_conv3d_ring(const uint16_t* __restrict__ x, const __grid_constant__ RingParams
         // straight-line path: no column predicates, row pointer carried from plane to plane.
         constexpr bool fast = FAST;      // host: ncols == CP, 32-byte aligned fp16 rows (ring_conv)
         uint32_t grp = 0, gphase = 0;
-        const bool late_release = RING_LATE_RELEASE && !(p.dbg & 16);      // ATVS_RING_DEBUG bit 16: release before the stores
-        TRACE_DECL
         UnitIter units(p);
         Unit un;
         while (units.next(p, un)) {
@@ -438,7 +384,6 @@ k_conv3d_ring(const uint16_t* __restrict__ x, const __grid_constant__ RingParams
             }
             for (int t = 0; t < un.zlen; ++t) {
                 mbar_wait(&tfull[grp], gphase);
-                TRACE(0);
                 tc_fence_after();
                 const uint32_t taddr = tmem_base + ((uint32_t)(g * 32) << 16) + grp * (uint32_t)CP;
                 uint64_t* const tempty_bar = &tempty[grp];
@@ -449,26 +394,18 @@ k_conv3d_ring(const uint16_t* __restrict__ x, const __grid_constant__ RingParams
 #pragma unroll
                     for (int c = 0; c < CP; c += 8) tc_ld8(taddr + (uint32_t)mt * Cfg::TILE_COLS + c, v[mt] + c);
                 tc_wait_ld();
-                TRACE(1);
-                if (!(p.dbg & 8)) {
 #pragma unroll
-                    for (int mt = 0; mt < RG_MT; ++mt)
+                for (int mt = 0; mt < RG_MT; ++mt)
 #pragma unroll
-                        for (int c = 0; c < CP; c += 8) tc_st8_zero(taddr + (uint32_t)mt * Cfg::TILE_COLS + c);
-                }
-                // the zeroing stores complete while this plane is converted and stored: the group is released after
-                // that (the accumulator ring has groups to spare), see release() below
-                auto release = [&]() {
-                    __syncwarp();          // rows outside the volume skipped the stores: reconverge before the aligned wait
-                    tc_wait_st();
-                    tc_fence_before();
-                    __syncwarp();
-                    if (lane == 0) mbar_arrive(tempty_bar);
-                };
-                if (!late_release) release();
-                TRACE(2);
-                TRACE_NEXT();
-                if (FAST && yok && !(p.dbg & 4)) {
+                    for (int c = 0; c < CP; c += 8) tc_st8_zero(taddr + (uint32_t)mt * Cfg::TILE_COLS + c);
+                // release the group before the plane is converted and stored (releasing it after the stores, with the
+                // zeroing overlapped with the conversion, measured 31.7 vs 31.9 us per 8 -> 8 layer in steady state)
+                __syncwarp();
+                tc_wait_st();
+                tc_fence_before();
+                __syncwarp();
+                if (lane == 0) mbar_arrive(tempty_bar);
+                if (FAST && yok) {
                     const int z = un.z0 + t;
                     const int zc = (z == 0) ? 0 : (z == p.D - 1 ? 2 : 1);
 #pragma unroll
@@ -510,7 +447,7 @@ k_conv3d_ring(const uint16_t* __restrict__ x, const __grid_constant__ RingParams
                             }
                         }
                     }
-                } else if (!FAST && yok && !(p.dbg & 4)) {
+                } else if (!FAST && yok) {
                 const int z = un.z0 + t;
                 const int zc = (z == 0) ? 0 : (z == p.D - 1 ? 2 : 1);
 #pragma unroll
@@ -548,10 +485,8 @@ k_conv3d_ring(const uint16_t* __restrict__ x, const __grid_constant__ RingParams
                 }
                 }
                 orow16 += zstride;
-                if (late_release) release();
             }
         }
-        if (warp == 5 && lane == 0) TRACE_DUMP("E");
         if (stats != nullptr) {
             // [sums | sums of squares] of this thread -> warp totals -> fp64 atomics
 #pragma unroll
@@ -607,27 +542,27 @@ __global__ void k_pack_ring(const float* __restrict__ w, int Cin, int Cout, int 
     }
 }
 
-template <int CIN, int CP, int MT, int MINB, bool FAST>
+template <int CIN, int CP, int MINB, bool FAST>
 int launch_ring1(const uint16_t* x, const RingParams& p, const uint8_t* wimg, float* out, double* stats,
                  const float* bias, size_t smem, int grid, cudaStream_t st) {
     static bool attr_set = false;
     if (!attr_set) {
-        ATVS_CUDA(cudaFuncSetAttribute(k_conv3d_ring<CIN, CP, MT, MINB, FAST>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+        ATVS_CUDA(cudaFuncSetAttribute(k_conv3d_ring<CIN, CP, MINB, FAST>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
         attr_set = true;
     }
-    k_conv3d_ring<CIN, CP, MT, MINB, FAST><<<grid, RG_THREADS, smem, st>>>(x, p, wimg, out, stats, bias);
+    k_conv3d_ring<CIN, CP, MINB, FAST><<<grid, RG_THREADS, smem, st>>>(x, p, wimg, out, stats, bias);
     ATVS_LAUNCH_CHECK();
     return 0;
 }
 
 // FAST epilogue: the slab fills its CP columns and the rows are saturated fp16 in whole, 32-byte aligned groups of 8
-template <int CIN, int CP, int MT, int MINB>
+template <int CIN, int CP, int MINB>
 int launch_ring(const uint16_t* x, const RingParams& p, const uint8_t* wimg, float* out, double* stats,
                 const float* bias, size_t smem, int grid, cudaStream_t st) {
     const bool fast = p.ncols == CP && p.raw16 && ((p.Cout | p.coff) & 7) == 0 && (((uintptr_t)out) & 31) == 0 &&
-                      (bias == nullptr || (((uintptr_t)bias) & 15) == 0) && !(p.dbg & 32);
-    return fast ? launch_ring1<CIN, CP, MT, MINB, true>(x, p, wimg, out, stats, bias, smem, grid, st)
-                : launch_ring1<CIN, CP, MT, MINB, false>(x, p, wimg, out, stats, bias, smem, grid, st);
+                      (bias == nullptr || (((uintptr_t)bias) & 15) == 0);
+    return fast ? launch_ring1<CIN, CP, MINB, true>(x, p, wimg, out, stats, bias, smem, grid, st)
+                : launch_ring1<CIN, CP, MINB, false>(x, p, wimg, out, stats, bias, smem, grid, st);
 }
 
 size_t ring_slab_bytes(int Cin, int cp) {
@@ -661,8 +596,7 @@ bool ring_applicable(int B, int D, int H, int W, int stride, int transposed) {
     // smaller volumes: the per-tap TMA kernel (conv_tc.cu).  Alone it is as fast there, but it fetches every input voxel 27
     // times through L2 and spends 5 x the SM time of the ring on a 32 -> 32 layer of 32x32x40 voxels: inside the step the
     // ring wins from ~32k voxels (5.21 -> 5.05 ms per cfg2 depth map with the threshold lowered from 65536)
-    const long long minvox = getenv("ATVS_RING_MINVOX") ? atoll(getenv("ATVS_RING_MINVOX")) : 32768;
-    return !transposed && stride == 1 && (long long)D * H * W >= minvox && H >= 8 && W >= 8;
+    return !transposed && stride == 1 && (long long)D * H * W >= 32768 && H >= 8 && W >= 8;
 }
 
 int ring_conv(const void* x16, int dtype, const void* wimg, int B, int D, int H, int W, int Cin, int Cout, float* raw_out,
@@ -676,19 +610,10 @@ int ring_conv(const void* x16, int dtype, const void* wimg, int B, int D, int H,
     p.raw16 = raw16;
     p.fmt = tc_fmt_bits(dtype);
     p.sat = raw16 ? atvs_sat_ptr() : nullptr;
-    // 4-tile planes for the 8-channel layers exist (ATVS_RING_MT=4) but measured no faster than 2-tile planes
-    // (profiles/r02_ring_probe.txt: 45 us either way at cfg2): the default stays 2
-    int mt = 2;
-    if (const char* e = getenv("ATVS_RING_MT")) mt = (atoi(e) == 4 && Cin == 8 && cp == 8 && W >= 32) ? 4 : 2;
-    p.TX = 8 * mt;
-    p.nXT = (W + p.TX - 1) / p.TX;
+    p.nXT = (W + RG_TX - 1) / RG_TX;
     p.nYT = (H + RG_TY - 1) / RG_TY;
     p.wbytes = (int)ring_slab_bytes(Cin, cp);
-    {
-        const char* e = getenv("ATVS_RING_DEBUG");
-        p.dbg = e ? atoi(e) : 0;
-    }
-    const size_t slot = ((size_t)(Cin / 8) * ((size_t)RG_HH * (p.TX + 2) * 16 + 16) + 127) / 128 * 128;
+    const size_t slot = ((size_t)(Cin / 8) * ((size_t)RG_HH * RG_WW * 16 + 16) + 127) / 128 * 128;
     const size_t fixed = 128 + (size_t)((p.wbytes + 127) & ~127) + (2 * RG_MAXR + 2 * RG_MAXG + 1) * 8 + 16;
     // two co-resident CTAs per SM when 2 x (weights + 4 planes) fit: their producer / MMA / epilogue
     // handshake latencies overlap
@@ -696,62 +621,18 @@ int ring_conv(const void* x16, int dtype, const void* wimg, int B, int D, int H,
     // small volumes: a second CTA per SM only halves the few plane steps each CTA gets, while every CTA pays
     // the same cold start (measured 41 -> 29 us for 16->16 on 64x64x80)
     if ((long long)B * p.nXT * p.nYT * D < (long long)sms * 2 * 12) minb = 1;
-    if (const char* e = getenv("ATVS_RING_MINB")) minb = atoi(e) == 1 ? 1 : minb;
     const size_t budget = (minb == 2 ? 110 : 220) * 1024;
     int nring = (int)((budget - fixed) / slot);
-    {
-        int cap = 8;
-        if (const char* e = getenv("ATVS_RING_R")) cap = atoi(e) < RG_MAXR ? (atoi(e) > 1 ? atoi(e) : 2) : RG_MAXR;
-        if (nring > cap) nring = cap;
-    }
+    if (nring > 8) nring = 8;
     if (nring < 2) {
         atvs_set_error("atvs_conv3d_bf16(ring): weights do not fit next to 2 ring planes (Cin=%d Cout=%d)", Cin, Cout);
         return ATVS_E_UNSUP;
     }
     p.nring = nring;
-    // planes per published group: 2 where a plane is small (Cin <= 16: the per-plane publish cost dominates), else 1
-    p.pg = 1;          // grouped publishing (ATVS_RING_PG=2..4) measured no faster: profiles/r02_ring_probe.txt
-    if (const char* e = getenv("ATVS_RING_PG")) p.pg = atoi(e) >= 1 && atoi(e) <= 4 ? atoi(e) : p.pg;
-    while (p.pg > 1 && 2 * p.pg + 1 > nring) --p.pg;
-    p.noinc = RING_NOINC_DEFAULT;
-    if (const char* e = getenv("ATVS_RING_NOINC")) p.noinc = atoi(e) != 0;
-    p.pf = (nring - 1) / p.pg;                      // groups in flight: pf * pg < nring keeps the ring deadlock-free
-    if (p.pf > 4) p.pf = 4;
-    if (const char* e = getenv("ATVS_RING_PF")) {
-        const int v = atoi(e);
-        if (v >= 1 && v * p.pg < nring) p.pf = v < 8 ? v : 8;
-    }
-    if (p.pf < 1) p.pf = 1;
-    {   // z segment length: minimise waves * (planes per unit)
-        const long long cols = (long long)B * p.nXT * p.nYT;
-        const long long slots = (long long)sms * minb;
-        // the MMA-bound wide-input layers (Cin >= 32: ~4x longer plane steps) weigh the startup less
-        int bz = ring_pick_zs(cols, D, slots, 1, 2, Cin >= 32 ? 0.8 : 0.4, Cin >= 32 ? 2.5 : 10.0, 4);
-        {   // experiment knobs: ATVS_RING_ZS_<Cin>_<Cout> (one layer kind) beats ATVS_RING_ZS (all)
-            char name[48];
-            snprintf(name, sizeof(name), "ATVS_RING_ZS_%d_%d", Cin, Cout);
-            const char* e = getenv(name);
-            if (!e) e = getenv("ATVS_RING_ZS");
-            if (e && atoi(e) > 0) bz = atoi(e) <= D ? atoi(e) : D;
-        }
-        p.ZS = bz;
-        p.nZS = (D + bz - 1) / bz;
-        p.nunits = cols * p.nZS;
-    }
+    p.pf = nring - 1 < 4 ? nring - 1 : 4;          // planes in flight: pf < nring keeps the ring deadlock-free
+    p.total = (long long)B * p.nXT * p.nYT * D;
     const size_t smem = fixed + (size_t)nring * slot;
-    int grid = (int)(p.nunits < (long long)sms * minb ? p.nunits : (long long)sms * minb);
-    {   // balanced plane ranges (default, ring_common.cuh); ATVS_RING_BALANCED=0: fixed z segments
-        p.total = (long long)B * p.nXT * p.nYT * D;
-        p.balanced = 1;
-        char name[48];
-        snprintf(name, sizeof(name), "ATVS_RING_BALANCED_%d_%d", Cin, Cout);
-        if (const char* e = getenv(name)) p.balanced = atoi(e) != 0;
-        else if (const char* e2 = getenv("ATVS_RING_BALANCED")) p.balanced = atoi(e2) != 0;
-        if (p.balanced) {
-            snprintf(name, sizeof(name), "ATVS_RING_CTAS_%d_%d", Cin, Cout);
-            grid = ring_balanced_grid(p.total, (long long)sms * minb, 12, 40, name, "ATVS_RING_CTAS");
-        }
-    }
+    const int grid = ring_balanced_grid(p.total, (long long)sms * minb, 12, 40);
     for (int slab = 0; slab < nslabs; ++slab) {
         p.coff = slab * cp;
         p.ncols = (Cout - p.coff < cp) ? Cout - p.coff : cp;
@@ -759,13 +640,9 @@ int ring_conv(const void* x16, int dtype, const void* wimg, int B, int D, int H,
         int rc = 0;
 #define RG_CASE(CI, CPV)                                                                                              \
     if (Cin == CI && cp == CPV) {                                                                                     \
-        rc = (minb == 2) ? launch_ring<CI, CPV, 2, 2>((const uint16_t*)x16, p, wi, raw_out, stats, bias, smem, grid, st) \
-                         : launch_ring<CI, CPV, 2, 1>((const uint16_t*)x16, p, wi, raw_out, stats, bias, smem, grid, st); \
+        rc = (minb == 2) ? launch_ring<CI, CPV, 2>((const uint16_t*)x16, p, wi, raw_out, stats, bias, smem, grid, st) \
+                         : launch_ring<CI, CPV, 1>((const uint16_t*)x16, p, wi, raw_out, stats, bias, smem, grid, st); \
     } else
-        if (Cin == 8 && cp == 8 && mt == 4) {
-            rc = (minb == 2) ? launch_ring<8, 8, 4, 2>((const uint16_t*)x16, p, wi, raw_out, stats, bias, smem, grid, st)
-                             : launch_ring<8, 8, 4, 1>((const uint16_t*)x16, p, wi, raw_out, stats, bias, smem, grid, st);
-        } else
         RG_CASE(8, 8) RG_CASE(8, 16) RG_CASE(8, 32) RG_CASE(16, 8) RG_CASE(16, 16) RG_CASE(16, 32)
         RG_CASE(32, 8) RG_CASE(32, 16) RG_CASE(32, 32) RG_CASE(64, 8) RG_CASE(64, 16) RG_CASE(64, 32)
         {

@@ -17,7 +17,6 @@
 #include "ring_common.cuh"
 #include "conv_ring.cuh"
 #include <cstring>
-#include <cstdlib>
 
 namespace {
 
@@ -37,22 +36,15 @@ struct S2Params {
     int raw16;                  // raw output dtype: 0 fp32, 1 saturated fp16
     uint32_t fmt;               // operand format bits of the instruction descriptor (tc_fmt_bits)
     unsigned long long* sat;    // saturation counter of the fp16 raw stores (atvs_sat_ptr)
-    int nXT, nYT, nZS, ZS;
+    int nXT, nYT;
     int nring;
     int wbytes;
-    int dbg;                    // ATVS_RING_DEBUG bit mask: 1 no loads, 2 no MMAs, 4 no stores (tools/steady_probe.py)
-    long long nunits;
-    int balanced;               // ring_common.cuh RingSpan: 1 = balanced ranges of output planes
-    long long total;            // tile columns * Do
+    long long total;            // tile columns * Do: the output plane sequence cut into one range per CTA (RingSpan)
 };
 
-// KPH: K phases of an input plane.  A ring slot holds CIN / KPH channels of the plane; the phases of a plane are staged
-// and multiplied one after the other into the same accumulators.  32 input channels as 2 phases of 16 halve the slot
-// (39 -> 20 KB), so that 4 slots + the weights fit two CTAs per SM (one CTA with ~190 KB of planes starves the passes
-// that share the SM: ATVS_RING_S2_MAXCIN history in DESIGN.md).
-template <int CIN, int CP, int KPH = 1>
+template <int CIN, int CP>
 struct S2Cfg {
-    static constexpr int NKC = CIN / 8 / KPH;                       // 8-channel chunks per slot
+    static constexpr int NKC = CIN / 8;                             // 8-channel chunks per slot
     static constexpr int SLOT_BYTES = (NKC * S2_PITCH + 127) / 128 * 128;
     static constexpr int NSTEPS = (CIN >= 16) ? 9 * (CIN / 16) : 5;
     static constexpr int NROWS = 3 * CP;
@@ -66,10 +58,10 @@ struct S2Unit {
 
 struct S2Iter {
     RingSpan span;
-    __device__ __forceinline__ explicit S2Iter(const S2Params& p) : span(p.balanced, p.total, p.nunits) {}
+    __device__ __forceinline__ explicit S2Iter(const S2Params& p) : span(p.total) {}
     __device__ __forceinline__ bool next(const S2Params& p, S2Unit& r) {
         long long t;
-        if (!span.next(p.balanced, p.Do, p.nZS, p.ZS, t, r.z0, r.zlen)) return false;
+        if (!span.next(p.Do, t, r.z0, r.zlen)) return false;
         r.x0 = (int)(t % p.nXT) * S2_TX;
         t /= p.nXT;
         r.y0 = (int)(t % p.nYT) * S2_TY;
@@ -92,13 +84,12 @@ __host__ __device__ constexpr uint32_t s2_tap_off(int tap) {
 __host__ __device__ constexpr int s2_pair_a(int s) { return s == 0 ? 0 : s == 1 ? 2 : s == 2 ? 5 : s == 3 ? 6 : 8; }
 __host__ __device__ constexpr int s2_pair_b(int s) { return s == 0 ? 1 : s == 1 ? 3 : s == 2 ? 4 : s == 3 ? 7 : 7; }
 
-template <int CIN, int CP, int MINB, int KPH>
+template <int CIN, int CP, int MINB>
 __global__ void __launch_bounds__(S2_THREADS, MINB)
 k_conv3d_ring_s2(const uint16_t* __restrict__ x, const __grid_constant__ S2Params p,
                  const uint8_t* __restrict__ wimg, float* __restrict__ out, double* __restrict__ stats,
                  const float* __restrict__ bias) {
-    using Cfg = S2Cfg<CIN, CP, KPH>;
-    static_assert(KPH == 1 || (CIN >= 32 && (CIN / 16) % KPH == 0), "K phases: whole K=16 steps");
+    using Cfg = S2Cfg<CIN, CP>;
     constexpr int G = S2_G;
 
     extern __shared__ uint8_t smem_raw[];
@@ -190,29 +181,26 @@ k_conv3d_ring_s2(const uint16_t* __restrict__ x, const __grid_constant__ S2Param
             }
             const uint16_t* zbase = x + ((size_t)un.b * p.D + 2 * un.z0) * zstride_in;
             for (int i = 0; i <= iend; ++i, zbase += zstride_in) {
+                mbar_wait(&empty[slot], sphase ^ 1);
+                const uint32_t dst0 = ring_u32 + slot * (uint32_t)Cfg::SLOT_BYTES;
 #pragma unroll
-                for (int h = 0; h < KPH; ++h) {            // phase h: channels [h * 8 NKC, (h + 1) * 8 NKC) of the plane
-                    mbar_wait(&empty[slot], sphase ^ 1);
-                    const uint32_t dst0 = ring_u32 + slot * (uint32_t)Cfg::SLOT_BYTES;
-#pragma unroll
-                    for (int k = 0; k < NITEM; ++k) {
-                        if (goff[k] != -2 && !(p.dbg & 1)) {
-                            const int j = ptid + k * S2_PRODUCERS;
-                            const int c = j % Cfg::NKC, v = j / Cfg::NKC;
-                            const int iy = v / S2_IW, ix = v - iy * S2_IW;
-                            const uint32_t soff = (uint32_t)(c * S2_PITCH +
-                                                             ((((iy & 1) << 1) | (ix & 1)) * S2_SUB + (iy >> 1) * S2_SC + (ix >> 1)) * 16);
-                            const bool ok = goff[k] >= 0;
-                            const uint16_t* src = ok ? zbase + goff[k] + h * (Cfg::NKC * 8) : x;
-                            asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst0 + soff), "l"(src),
-                                         "r"(ok ? 16 : 0)
-                                         : "memory");
-                        }
+                for (int k = 0; k < NITEM; ++k) {
+                    if (goff[k] != -2) {
+                        const int j = ptid + k * S2_PRODUCERS;
+                        const int c = j % Cfg::NKC, v = j / Cfg::NKC;
+                        const int iy = v / S2_IW, ix = v - iy * S2_IW;
+                        const uint32_t soff = (uint32_t)(c * S2_PITCH +
+                                                         ((((iy & 1) << 1) | (ix & 1)) * S2_SUB + (iy >> 1) * S2_SC + (ix >> 1)) * 16);
+                        const bool ok = goff[k] >= 0;
+                        const uint16_t* src = ok ? zbase + goff[k] : x;
+                        asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst0 + soff), "l"(src),
+                                     "r"(ok ? 16 : 0)
+                                     : "memory");
                     }
-                    asm volatile("cp.async.commit_group;" ::: "memory");
-                    if (++slot == (uint32_t)R) { slot = 0; sphase ^= 1; }
-                    if (++pending >= (uint32_t)PF) publish(PF - 1);
                 }
+                asm volatile("cp.async.commit_group;" ::: "memory");
+                if (++slot == (uint32_t)R) { slot = 0; sphase ^= 1; }
+                if (++pending >= (uint32_t)PF) publish(PF - 1);
             }
         }
         publish(0);
@@ -226,21 +214,15 @@ k_conv3d_ring_s2(const uint16_t* __restrict__ x, const __grid_constant__ S2Param
             constexpr uint32_t A_LBO = (CIN >= 16) ? ((uint32_t)(S2_PITCH >> 4) << 16) : 0u;
             const uint32_t a_lo_ring = (smem_u32(ring) >> 4) | A_LBO;
             const uint32_t b_lo0 = (smem_u32(wsm) >> 4) | ((uint32_t)((Cfg::NROWS * 16) >> 4) << 16);
-            // the MMAs of phase h of a plane: K=16 steps ks in [h * KS / KPH, (h + 1) * KS / KPH) of every in-plane tap; the
-            // slot holds the phase's chunks from 0, the weight image holds all steps (tap-major)
-            auto issue_plane = [&](uint32_t dcol, uint32_t a_lo0, uint32_t b_lo, uint32_t idesc, int h) {
+            auto issue_plane = [&](uint32_t dcol, uint32_t a_lo0, uint32_t b_lo, uint32_t idesc) {
                 constexpr int KS = (CIN >= 16) ? CIN / 16 : 1;
-                constexpr int KSP = KS / KPH > 0 ? KS / KPH : 1;
 #pragma unroll
-                for (int sl = 0; sl < Cfg::NSTEPS / KPH; ++sl) {
+                for (int s = 0; s < Cfg::NSTEPS; ++s) {
                     uint32_t aoff;
-                    int s;
                     if (CIN >= 16) {
-                        const int tp = sl / KSP, ksl = sl % KSP;
-                        s = tp * KS + h * KSP + ksl;
-                        aoff = (uint32_t)((2 * ksl * S2_PITCH) >> 4) + (s2_tap_off(tp) >> 4);
+                        const int tp = s / KS, ks = s % KS;
+                        aoff = (uint32_t)((2 * ks * S2_PITCH) >> 4) + (s2_tap_off(tp) >> 4);
                     } else {
-                        s = sl;
                         const uint32_t offa = s2_tap_off(s2_pair_a(s)), offb = s2_tap_off(s2_pair_b(s));
                         aoff = (offa >> 4) | (((offb - offa) >> 4) << 16);
                     }
@@ -267,27 +249,23 @@ k_conv3d_ring_s2(const uint16_t* __restrict__ x, const __grid_constant__ S2Param
                         if (++gw == (uint32_t)G) { gw = 0; gwphase ^= 1; }
                     }
                     const uint32_t gprev = (gcur == 0) ? (uint32_t)G - 1 : gcur - 1;
-#pragma unroll
-                    for (int h = 0; h < KPH; ++h) {
                     mbar_wait(&full[slot], sphase);
                     tc_fence_after();
                     const uint32_t a_lo0 = a_lo_ring + slot * (uint32_t)(Cfg::SLOT_BYTES >> 4);
-                    if (p.dbg & 2) {
-                    } else if (!even) {
-                        issue_plane(tmem_base + gcur * (uint32_t)CP, a_lo0, b_lo0 + ((W_W1 * 16u) >> 4), ring_idesc(CP) | p.fmt, h);
+                    if (!even) {
+                        issue_plane(tmem_base + gcur * (uint32_t)CP, a_lo0, b_lo0 + ((W_W1 * 16u) >> 4), ring_idesc(CP) | p.fmt);
                     } else if (j == 0) {
-                        issue_plane(tmem_base + gcur * (uint32_t)CP, a_lo0, b_lo0 + ((W_W0 * 16u) >> 4), ring_idesc(CP) | p.fmt, h);
+                        issue_plane(tmem_base + gcur * (uint32_t)CP, a_lo0, b_lo0 + ((W_W0 * 16u) >> 4), ring_idesc(CP) | p.fmt);
                     } else if (j >= un.zlen) {
-                        issue_plane(tmem_base + gprev * (uint32_t)CP, a_lo0, b_lo0 + ((W_W2W0 * 16u) >> 4), ring_idesc(CP) | p.fmt, h);
+                        issue_plane(tmem_base + gprev * (uint32_t)CP, a_lo0, b_lo0 + ((W_W2W0 * 16u) >> 4), ring_idesc(CP) | p.fmt);
                     } else if (gcur != 0) {
-                        issue_plane(tmem_base + gprev * (uint32_t)CP, a_lo0, b_lo0 + ((W_W2W0 * 16u) >> 4), ring_idesc(2 * CP) | p.fmt, h);
+                        issue_plane(tmem_base + gprev * (uint32_t)CP, a_lo0, b_lo0 + ((W_W2W0 * 16u) >> 4), ring_idesc(2 * CP) | p.fmt);
                     } else {                           // the pair wraps around the accumulator ring
-                        issue_plane(tmem_base + gprev * (uint32_t)CP, a_lo0, b_lo0 + ((W_W2W0 * 16u) >> 4), ring_idesc(CP) | p.fmt, h);
-                        issue_plane(tmem_base, a_lo0, b_lo0 + ((W_W0 * 16u) >> 4), ring_idesc(CP) | p.fmt, h);
+                        issue_plane(tmem_base + gprev * (uint32_t)CP, a_lo0, b_lo0 + ((W_W2W0 * 16u) >> 4), ring_idesc(CP) | p.fmt);
+                        issue_plane(tmem_base, a_lo0, b_lo0 + ((W_W0 * 16u) >> 4), ring_idesc(CP) | p.fmt);
                     }
                     tc_commit(&empty[slot]);
                     if (++slot == (uint32_t)R) { slot = 0; sphase ^= 1; }
-                    }
                     // output planes whose last contribution this was
                     const int tlast = (i == iend) ? un.zlen - 1 : (even ? j - 1 : -1);
                     while (tdone <= tlast) {
@@ -335,7 +313,7 @@ k_conv3d_ring_s2(const uint16_t* __restrict__ x, const __grid_constant__ S2Param
                 tc_fence_before();
                 __syncwarp();
                 if (lane == 0) mbar_arrive(tempty_bar);
-                if (!valid || (p.dbg & 4)) continue;
+                if (!valid) continue;
                 const size_t ooff = obase + (size_t)t * zstride;
                 if (bias != nullptr) {
                     // depth-invariant part of the layer (the tiled reference-feature half of the cost volume)
@@ -410,15 +388,15 @@ __global__ void k_pack_ring_s2(const float* __restrict__ w, int Cin, int Cout, i
     }
 }
 
-template <int CIN, int CP, int MINB, int KPH = 1>
+template <int CIN, int CP, int MINB>
 int launch_s2(const uint16_t* x, const S2Params& p, const uint8_t* wimg, float* out, double* stats,
               const float* bias, size_t smem, int grid, cudaStream_t st) {
     static bool attr_set = false;
     if (!attr_set) {
-        ATVS_CUDA(cudaFuncSetAttribute(k_conv3d_ring_s2<CIN, CP, MINB, KPH>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+        ATVS_CUDA(cudaFuncSetAttribute(k_conv3d_ring_s2<CIN, CP, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
         attr_set = true;
     }
-    k_conv3d_ring_s2<CIN, CP, MINB, KPH><<<grid, S2_THREADS, smem, st>>>(x, p, wimg, out, stats, bias);
+    k_conv3d_ring_s2<CIN, CP, MINB><<<grid, S2_THREADS, smem, st>>>(x, p, wimg, out, stats, bias);
     ATVS_LAUNCH_CHECK();
     return 0;
 }
@@ -428,7 +406,10 @@ size_t s2_slab_bytes(int Cin, int cp) { return (size_t)ring_nsteps(Cin) * 2 * 3 
 
 }  // namespace
 
-bool ring_s2_supported(int Cin, int Cout) { return (Cin == 8 || Cin == 16 || Cin == 32) && Cout >= 1 && Cout <= 64; }
+// Cin = 32 needs ~200 KB of ring planes per CTA (or two K phases of 16 channels per plane to fit two CTAs per SM):
+// standalone it beats the per-tap TMA kernel (73 vs 88 us at cfg2), but it monopolises the SM while the other streams
+// of a step want to co-run (measured +0.25 ms per depth map), so the 32-channel layers stay on the per-tap kernel
+bool ring_s2_supported(int Cin, int Cout) { return (Cin == 8 || Cin == 16) && Cout >= 1 && Cout <= 64; }
 
 size_t ring_s2_weight_bytes(int Cin, int Cout) {
     if (!ring_s2_supported(Cin, Cout)) return 0;
@@ -444,18 +425,11 @@ int ring_s2_pack(const float* kernel, int Cin, int Cout, int dtype, void* wimg, 
     return 0;
 }
 
-#ifndef RING_S2_MINVOX
-#define RING_S2_MINVOX 32768       // output voxels from which the plane ring replaces the per-tap TMA kernel (131072 -> 32768: 5.03 -> 5.00 ms per cfg2 depth map)
-#endif
+// output voxels from which the plane ring replaces the per-tap TMA kernel (131072 -> 32768: 5.03 -> 5.00 ms per cfg2
+// depth map)
+constexpr long long RING_S2_MINVOX = 32768;
 bool ring_s2_applicable(int B, int D, int H, int W, int Cin, int Cout) {
-    // Cin = 32 needs ~200 KB of ring planes per CTA: standalone it beats the per-tap TMA kernel (73 vs 88 us
-    // at cfg2), but it monopolises the SM while the other streams of a step want to co-run (measured
-    // +0.25 ms per depth map), so it is opt-in (ATVS_RING_S2_MAXCIN=32)
-    const char* e = getenv("ATVS_RING_S2_MAXCIN");
-    if (Cin > (e ? atoi(e) : 16)) return false;
-    const long long minvox = getenv("ATVS_RING_S2_MINVOX") ? atoll(getenv("ATVS_RING_S2_MINVOX")) : RING_S2_MINVOX;
-    return ring_s2_supported(Cin, Cout) && ((D | H | W) & 1) == 0 && (long long)(D / 2) * (H / 2) * (W / 2) >= minvox &&
-           getenv("ATVS_NO_RING_S2") == nullptr;
+    return ring_s2_supported(Cin, Cout) && ((D | H | W) & 1) == 0 && (long long)(D / 2) * (H / 2) * (W / 2) >= RING_S2_MINVOX;
 }
 
 int ring_s2_conv(const void* x16, int dtype, const void* wimg, int B, int D, int H, int W, int Cin, int Cout, float* raw_out,
@@ -472,54 +446,20 @@ int ring_s2_conv(const void* x16, int dtype, const void* wimg, int B, int D, int
     p.nXT = (p.Wo + S2_TX - 1) / S2_TX;
     p.nYT = (p.Ho + S2_TY - 1) / S2_TY;
     p.wbytes = (int)s2_slab_bytes(Cin, cp);
-    {
-        const char* e = getenv("ATVS_RING_DEBUG");
-        p.dbg = e ? atoi(e) : 0;
-    }
-    // 32 input channels: two K phases of 16 per plane (S2Cfg) unless ATVS_S2_KPH=1
-    int kph = Cin == 32 ? 2 : 1;
-    if (const char* e = getenv("ATVS_S2_KPH")) kph = (Cin == 32 && atoi(e) == 2) ? 2 : 1;
-    const size_t slot = ((size_t)(Cin / 8 / kph) * S2_PITCH + 127) / 128 * 128;
+    const size_t slot = ((size_t)(Cin / 8) * S2_PITCH + 127) / 128 * 128;
     const size_t fixed = 128 + (size_t)((p.wbytes + 127) & ~127) + (2 * 8 + 2 * S2_G + 1) * 8 + 16;
-    int minb = (cp < 32 && fixed + 4 * slot <= 110 * 1024) ? 2 : 1;
-    if (const char* e = getenv("ATVS_RING_MINB")) minb = atoi(e) == 1 ? 1 : minb;
+    const int minb = (cp < 32 && fixed + 4 * slot <= 110 * 1024) ? 2 : 1;
     const size_t budget = (minb == 2 ? 110 : 220) * 1024;
     int nring = (int)((budget - fixed) / slot);
     if (nring > 8) nring = 8;
-    if (const char* e = getenv("ATVS_RING_R")) nring = atoi(e) < nring ? atoi(e) : nring;
-    if (const char* e = getenv("ATVS_S2_R")) nring = atoi(e) < nring && atoi(e) >= 2 ? atoi(e) : nring;
     if (nring < 2) {
         atvs_set_error("atvs_conv3d_bf16(ring s2): weights do not fit next to 2 ring planes (Cin=%d Cout=%d)", Cin, Cout);
         return ATVS_E_UNSUP;
     }
     p.nring = nring;
-    {   // output z segment length: minimise waves * (input planes per unit)
-        const long long cols = (long long)B * p.nXT * p.nYT;
-        const long long slots = (long long)sms * minb;
-        int bz = ring_pick_zs(cols, p.Do, slots, 2, 1, Cin >= 32 ? 0.8 : 0.4, Cin >= 32 ? 2.5 : 10.0, 2);
-        {   // experiment knobs: ATVS_S2_ZS_<Cin>_<Cout> (one layer kind) beats ATVS_S2_ZS (all stride-2 ring layers)
-            char name[48];
-            snprintf(name, sizeof(name), "ATVS_S2_ZS_%d_%d", Cin, Cout);
-            const char* e = getenv(name);
-            if (!e) e = getenv("ATVS_S2_ZS");
-            if (e && atoi(e) > 0) bz = atoi(e) <= p.Do ? atoi(e) : p.Do;
-        }
-        p.ZS = bz;
-        p.nZS = (p.Do + bz - 1) / bz;
-        p.nunits = cols * p.nZS;
-    }
+    p.total = (long long)B * p.nXT * p.nYT * p.Do;
     const size_t smem = fixed + (size_t)nring * slot;
-    int grid = (int)(p.nunits < (long long)sms * minb ? p.nunits : (long long)sms * minb);
-    {   // balanced ranges of output planes (default, ring_common.cuh); ATVS_S2_BALANCED=0: fixed z segments
-        p.total = (long long)B * p.nXT * p.nYT * p.Do;
-        p.balanced = 1;
-        if (const char* e = getenv("ATVS_S2_BALANCED")) p.balanced = atoi(e) != 0;
-        if (p.balanced) {
-            char name[48];
-            snprintf(name, sizeof(name), "ATVS_S2_CTAS_%d_%d", Cin, Cout);
-            grid = ring_balanced_grid(p.total, (long long)sms * minb, 20, 80, name, "ATVS_S2_CTAS");
-        }
-    }
+    const int grid = ring_balanced_grid(p.total, (long long)sms * minb, 20, 80);
     for (int slab = 0; slab < nslabs; ++slab) {
         p.coff = slab * cp;
         p.ncols = (Cout - p.coff < cp) ? Cout - p.coff : cp;
@@ -530,14 +470,7 @@ int ring_s2_conv(const void* x16, int dtype, const void* wimg, int B, int D, int
         rc = (minb == 2) ? launch_s2<CI, CPV, 2>((const uint16_t*)x16, p, wi, raw_out, stats, bias, smem, grid, st) \
                          : launch_s2<CI, CPV, 1>((const uint16_t*)x16, p, wi, raw_out, stats, bias, smem, grid, st); \
     } else
-        if (Cin == 32 && kph == 2 && cp == 16) {
-            rc = (minb == 2) ? launch_s2<32, 16, 2, 2>((const uint16_t*)x16, p, wi, raw_out, stats, bias, smem, grid, st)
-                             : launch_s2<32, 16, 1, 2>((const uint16_t*)x16, p, wi, raw_out, stats, bias, smem, grid, st);
-        } else if (Cin == 32 && kph == 2 && cp == 32) {
-            rc = (minb == 2) ? launch_s2<32, 32, 2, 2>((const uint16_t*)x16, p, wi, raw_out, stats, bias, smem, grid, st)
-                             : launch_s2<32, 32, 1, 2>((const uint16_t*)x16, p, wi, raw_out, stats, bias, smem, grid, st);
-        } else
-        S2_CASE(8, 16) S2_CASE(8, 32) S2_CASE(16, 16) S2_CASE(16, 32) S2_CASE(32, 16) S2_CASE(32, 32)
+        S2_CASE(8, 16) S2_CASE(8, 32) S2_CASE(16, 16) S2_CASE(16, 32)
         {
             atvs_set_error("atvs_conv3d_bf16(ring s2): no kernel for Cin=%d CP=%d", Cin, cp);
             return ATVS_E_UNSUP;

@@ -338,9 +338,6 @@ extern "C" size_t atvs_packed_weight_bytes(int Cin, int Cout, int transposed) {
     return bytes;
 }
 
-#ifndef TC_SHARED_MINTILES
-#define TC_SHARED_MINTILES 4      // whole cfg2 step: 5.51 (1) 5.47 (2) 5.45 (4) 5.45 (6) 5.47 (8) 5.71 ms (12)
-#endif
 static size_t tap_image_bytes(int Cin, int Cout, int transposed) {
     const SlabPlan sp = plan_slabs(Cin, Cout, transposed ? 8 : 27);
     size_t elems = 0;
@@ -352,13 +349,10 @@ static size_t tap_image_bytes(int Cin, int Cout, int transposed) {
 // CTAs of a per-tap launch.  Every CTA pays a fixed cost (TMEM allocation, all taps' weights into shared memory, pipeline
 // fill) worth several tiles; a launch that owns the GPU wants one CTA per SM, but in a step whose passes share the SMs
 // (atvs_set_concurrency > 1) fewer CTAs with more tiles each spend less SM time on the same work.
-// ATVS_TC_MINTILES: tiles per CTA when the SMs are shared.
+// Tiles per CTA when the SMs are shared, whole cfg2 step: 5.51 (1) 5.47 (2) 5.45 (4) 5.45 (6) 5.47 (8) 5.71 ms (12).
+constexpr int TC_SHARED_MINTILES = 4;
 static int tc_grid(long long nwork, int sms) {
-    int mint = 1;
-    if (atvs_concurrency() > 1) {
-        mint = TC_SHARED_MINTILES;
-        if (const char* e = getenv("ATVS_TC_MINTILES")) mint = atoi(e) > 0 ? atoi(e) : mint;
-    }
+    const int mint = atvs_concurrency() > 1 ? TC_SHARED_MINTILES : 1;
     long long g = nwork / mint;
     if (g < 1) g = 1;
     if (g > sms) g = sms;

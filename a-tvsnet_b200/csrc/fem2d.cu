@@ -8,14 +8,6 @@
 // fp32 CUDA-core kernels (register-tiled direct convolution): the PARITY path of this row.  The tensor-core (tcgen05)
 // version - channel-chunked taps, dilation, bias/ReLU epilogue - is the next step; see DESIGN.md section 6.
 #include "common.cuh"
-#include <cstdlib>
-
-#ifndef C2_MINB
-#define C2_MINB 3
-#endif
-#ifndef C2_FFMA2
-#define C2_FFMA2 1
-#endif
 
 namespace {
 
@@ -27,33 +19,31 @@ struct Conv2dParams {
 
 // d0 += a.x * b.x, d1 += a.y * b.y as ONE fma.rn.f32x2 (sm_100 FFMA2)
 __device__ __forceinline__ void ffma2(float& d0, float& d1, float2 a, float2 b) {
-#if C2_FFMA2
     unsigned long long d, ua, ub;
     asm("mov.b64 %0, {%1, %2};" : "=l"(d) : "f"(d0), "f"(d1));
     asm("mov.b64 %0, {%1, %2};" : "=l"(ua) : "f"(a.x), "f"(a.y));
     asm("mov.b64 %0, {%1, %2};" : "=l"(ub) : "f"(b.x), "f"(b.y));
     asm("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(d) : "l"(ua), "l"(ub));
     asm("mov.b64 {%0, %1}, %2;" : "=f"(d0), "=f"(d1) : "l"(d));
-#else
-    d0 = fmaf(a.x, b.x, d0);
-    d1 = fmaf(a.y, b.y, d1);
-#endif
 }
 
 constexpr int C2_TH = 8, C2_CO = 32, C2_KC = 32;      // tile: 8 rows x (8 * PX) pixels, 32 output channels, 32-channel K steps
+constexpr int C2_CT = C2_CO / 4;                        // output channels per thread
 constexpr int C2_WPT = C2_KC * C2_CO / 256;             // weights per thread and K step
+constexpr int C2_MINB = 3;                              // blocks per SM
 constexpr int C2_UNROLL = 8;                            // all 8 four-channel sub-steps of a K step unrolled: 20.7 ms per cfg2 frame (4: 22.3)
 
 // block = 256 threads = 64 pixel groups (PX consecutive x) x 4 groups of 8 output channels; one 8 x (8*PX) pixel tile
 // and 32 output channels per block.  Per (tap, 16-channel chunk) the weights [16][32] are staged in shared memory; a
 // thread does PX*32 FMAs per PX input float4 loads and 8 weight LDS.128.  PX = 4 for the large maps, PX = 2 when that
 // would leave the SMs with about one block each (the 1/4-resolution layers: occupancy 14 % with PX = 4).
-template <int K, int PX, int CT>
-__global__ void __launch_bounds__(256, CT == 16 ? 1 : C2_MINB)
+// 16 output channels per thread (64 per block: each loaded input pixel feeds twice the FMAs) were measured at cfg2 (5 views
+// batched): 23.9 ms per frame against 20.7 with 8 (168 registers: one block per SM).
+template <int K, int PX>
+__global__ void __launch_bounds__(256, C2_MINB)
 k_conv2d_fp32(const float* __restrict__ x, const float* __restrict__ w, const float* __restrict__ bias,
               const Conv2dParams p, float* __restrict__ out) {
-    constexpr int CO = 4 * CT;                               // output channels per block: 4 thread groups x CT
-    constexpr int WPT = C2_KC * CO / 256;
+    constexpr int CT = C2_CT, CO = C2_CO, WPT = C2_WPT;
     __shared__ __align__(16) float ws[2][C2_KC][CO];         // double buffered: ONE barrier per K step
     const int t = threadIdx.x;
     const int cg = t & 3, q = t >> 2;
@@ -357,25 +347,17 @@ extern "C" int atvs_conv2d_fp32(const float* x, const float* kernel, const float
     p.B = B; p.H = H; p.W = W; p.Cin = Cin; p.Cout = Cout; p.Ho = Ho; p.Wo = Wo;
     p.stride = stride; p.rate = rate; p.pad_t = pad_top; p.pad_l = pad_left; p.relu = relu;
     p.tiles_y = (Ho + C2_TH - 1) / C2_TH;
-    // 16 output channels per thread (64 per block) where the layer has them and the grid still fills the SMs: the input
-    // pixel a thread loads then feeds twice the FMAs (ATVS_FEM_CT=8 forces the 8-channel tile)
-    int ct = 8;      // measured at cfg2 (5 views batched): 20.7 ms per frame with 8 channels per thread, 23.9 with 16 (168 registers: one block per SM)
-    if (const char* e = getenv("ATVS_FEM_CT")) ct = (atoi(e) == 16 && Cout % 64 == 0) ? 16 : (atoi(e) == 8 ? 8 : ct);
-    if (ct == 16 && (long long)B * ((Wo + 31) / 32) * p.tiles_y * (Cout / 64) < 3LL * atvs_num_sms()) ct = 8;
-    const int slabs = (Cout + 4 * ct - 1) / (4 * ct);
+    const int slabs = (Cout + C2_CO - 1) / C2_CO;
     // 4 pixels per thread unless that leaves fewer than ~4 blocks per SM
     int px = 4;
     if ((long long)B * ((Wo + 31) / 32) * p.tiles_y * slabs < 3LL * atvs_num_sms()) px = 2;
     p.tiles_x = (Wo + 8 * px - 1) / (8 * px);
     dim3 grid((unsigned)((long long)B * p.tiles_x * p.tiles_y), (unsigned)slabs);
     cudaStream_t st = (cudaStream_t)stream;
-    if (ct == 16) {
-        if (ksize == 1) k_conv2d_fp32<1, 4, 16><<<grid, 256, 0, st>>>(x, kernel, bias, p, out);
-        else k_conv2d_fp32<3, 4, 16><<<grid, 256, 0, st>>>(x, kernel, bias, p, out);
-    } else if (ksize == 1 && px == 4) k_conv2d_fp32<1, 4, 8><<<grid, 256, 0, st>>>(x, kernel, bias, p, out);
-    else if (ksize == 1) k_conv2d_fp32<1, 2, 8><<<grid, 256, 0, st>>>(x, kernel, bias, p, out);
-    else if (px == 4) k_conv2d_fp32<3, 4, 8><<<grid, 256, 0, st>>>(x, kernel, bias, p, out);
-    else k_conv2d_fp32<3, 2, 8><<<grid, 256, 0, st>>>(x, kernel, bias, p, out);
+    if (ksize == 1 && px == 4) k_conv2d_fp32<1, 4><<<grid, 256, 0, st>>>(x, kernel, bias, p, out);
+    else if (ksize == 1) k_conv2d_fp32<1, 2><<<grid, 256, 0, st>>>(x, kernel, bias, p, out);
+    else if (px == 4) k_conv2d_fp32<3, 4><<<grid, 256, 0, st>>>(x, kernel, bias, p, out);
+    else k_conv2d_fp32<3, 2><<<grid, 256, 0, st>>>(x, kernel, bias, p, out);
     ATVS_LAUNCH_CHECK();
     return 0;
 }

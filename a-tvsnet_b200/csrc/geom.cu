@@ -303,10 +303,7 @@ __device__ __forceinline__ void store4(__half* p, float4 v) {
     __stcs(reinterpret_cast<uint2*>(p), pk);
 }
 
-#ifndef ATVS_K1_DCHUNK
-#define ATVS_K1_DCHUNK 8      // depth planes per block of K1 (measured: 4 / 8 / 16, see DESIGN.md)
-#endif
-constexpr int K1_DCHUNK = ATVS_K1_DCHUNK;
+constexpr int K1_DCHUNK = 8;      // depth planes per block of K1 (measured: 4 / 8 / 16, see DESIGN.md)
 
 // grid: x = pixel*channel-group tiles, y = depth chunks, z = batch.
 // one thread = one pixel x 4 channels, looping over K1_DCHUNK planes with the reference
@@ -1233,7 +1230,7 @@ extern "C" int atvs_build_cost_volume(const float* ref_feature, const float* vie
         return launch_k1<float>(ref_feature, view_feature, homographies, ref_homographies, B, D, h, w, F, mode,
                                 (float*)out, st);
     const bool half_out = out_dtype == ATVS_BF16 || out_dtype == ATVS_F16;
-    if (half_out && !ref_homographies && k1_h_supported(F) && getenv("ATVS_K1_F32SRC") == nullptr) {
+    if (half_out && !ref_homographies && k1_h_supported(F)) {
         // 16-bit volume: gather from a 16-bit copy of the source feature map (stream-ordered scratch)
         uint16_t* vb = nullptr;
         const long long n = (long long)B * h * w * F;
@@ -1296,7 +1293,7 @@ extern "C" int atvs_prob2depth(const float* prob_volume, int B, int D, int H, in
     {
         const int Ho = H * 4;
         const long long blocks = (long long)B * Ho * ((W + 31) / 32);
-        if (blocks <= 0x7fffffffLL && getenv("ATVS_K4_SIMPLE") == nullptr)
+        if (blocks <= 0x7fffffffLL)
             k_prob2depth_up_sliced<4><<<(unsigned)blocks, 256, 0, st>>>(prob_volume, B, D, H, W, depth_start, depth_interval,
                                                                        depth, prob_map);
         else

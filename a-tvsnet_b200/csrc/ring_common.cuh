@@ -1,20 +1,6 @@
 // ring_common.cuh - helpers shared by the halo-ring convolution kernels (conv_ring.cu, conv_ring_s2.cu)
 #pragma once
 #include "tc_ptx.cuh"
-#include <cstdlib>
-
-// per-role clock64 timelines of CTA 0 (build with -DATVS_RING_TRACE: tools/build_trace.sh, tools/ring_trace.py)
-#ifdef ATVS_RING_TRACE
-#define TRACE_DECL long long tr_[3][48]; int trn_ = 0; for (int q_ = 0; q_ < 48; ++q_) tr_[0][q_] = tr_[1][q_] = tr_[2][q_] = 0;
-#define TRACE(k) do { if (blockIdx.x == 0 && trn_ < 48) tr_[k][trn_] = clock64(); } while (0)
-#define TRACE_NEXT() do { ++trn_; } while (0)
-#define TRACE_DUMP(name) do { if (blockIdx.x == 0) for (int q_ = 0; q_ < 48 && q_ < trn_; ++q_) printf("%s %d %lld %lld %lld\n", name, q_, tr_[0][q_], tr_[1][q_], tr_[2][q_]); } while (0)
-#else
-#define TRACE_DECL
-#define TRACE(k)
-#define TRACE_NEXT()
-#define TRACE_DUMP(name)
-#endif
 
 namespace {
 
@@ -78,38 +64,24 @@ __host__ __device__ constexpr uint32_t ring_idesc(int n) {
 }
 
 
-// Work of one CTA of a plane-ring kernel as a sequence of units (tile column, z0, zlen).
-//   fixed z segments (balanced = 0): units u = blockIdx.x, blockIdx.x + gridDim.x, ... of length ZS.  The tile columns
-//     of a volume rarely divide by the resident CTAs (cfg2: 80 columns x 5 segments = 400 units on 296 CTAs = 1.35
-//     waves: the launch lasts 2 x 28 plane steps where 37 would do).
-//   balanced = 1 (default): the planes of all columns form ONE sequence (column-major, z fastest) that is cut into
-//     gridDim.x equal ranges; a range that crosses a column end becomes two units.  Every CTA runs total/grid planes
-//     (+ the halo planes of its 1-2 units), whatever the volume.
+// Work of one CTA of a plane-ring kernel as a sequence of units (tile column, z0, zlen): the planes of all columns form
+// ONE sequence (column-major, z fastest) that is cut into gridDim.x equal ranges; a range that crosses a column end
+// becomes two units.  Every CTA runs total/grid planes (+ the halo planes of its 1-2 units), whatever the volume.
+// (Fixed z segments per CTA, measured before: the tile columns of a volume rarely divide by the resident CTAs - cfg2:
+// 80 columns x 5 segments = 400 units on 296 CTAs = 1.35 waves, the launch lasts 2 x 28 plane steps where 37 would do.)
 struct RingSpan {
     long long pos, end;
-    __device__ __forceinline__ RingSpan(int balanced, long long total, long long nunits) {
-        if (balanced) {
-            pos = total * (long long)blockIdx.x / (long long)gridDim.x;
-            end = total * ((long long)blockIdx.x + 1) / (long long)gridDim.x;
-        } else {
-            pos = blockIdx.x;
-            end = nunits;
-        }
+    __device__ __forceinline__ explicit RingSpan(long long total) {
+        pos = total * (long long)blockIdx.x / (long long)gridDim.x;
+        end = total * ((long long)blockIdx.x + 1) / (long long)gridDim.x;
     }
-    // next unit: balanced -> (col, z0, zlen) of the piece; fixed segments -> (col, z0, zlen) of unit `pos`
-    __device__ __forceinline__ bool next(int balanced, int nz, int nZS, int ZS, long long& col, int& z0, int& zlen) {
+    // next unit: (col, z0, zlen) of the next piece of the range
+    __device__ __forceinline__ bool next(int nz, long long& col, int& z0, int& zlen) {
         if (pos >= end) return false;
-        if (balanced) {
-            col = pos / nz;
-            z0 = (int)(pos - col * nz);
-            zlen = (int)min((long long)(nz - z0), end - pos);
-            pos += zlen;
-        } else {
-            col = pos / nZS;
-            z0 = (int)(pos - col * nZS) * ZS;
-            zlen = min(ZS, nz - z0);
-            pos += gridDim.x;
-        }
+        col = pos / nz;
+        z0 = (int)(pos - col * nz);
+        zlen = (int)min((long long)(nz - z0), end - pos);
+        pos += zlen;
         return true;
     }
 };
@@ -118,48 +90,22 @@ struct RingSpan {
 // allocation, weight image, pipeline fill, cold first loads) is worth ~10 plane steps, and a tensor CTA holds half an
 // SM's shared memory and TMEM columns while it lives.  A launch that has the GPU to itself wants many CTAs
 // (`alone` planes per CTA); in a step of 8 passes on 8 streams FEWER, LONGER CTAs win (`shared` planes per CTA:
-// tools/tune_step.py on cfg2, profiles/r02_tune_step_balanced.txt - 5.95 ms with fixed z segments, 6.46 with 12 planes
+// profiles/r02_tune_step_balanced.txt on cfg2 - 5.95 ms with fixed z segments, 6.46 with 12 planes
 // per CTA everywhere, 5.60 with 40 (stride 1) / 80 (stride 2) / 160 (transposed)), at the price of the launch's own
 // latency (a 16-CTA transposed convolution lasts 95 us instead of 33).  The caller says how many passes it runs side
 // by side (atvs_set_concurrency, 1 by default); in between the two settings are interpolated.
-// `knob1/knob2` (environment, optional) set the CTA count; ATVS_RING_MINPLANES overrides the planes per CTA.
-inline int ring_balanced_grid(long long total, long long slots, int alone, int shared, const char* knob1, const char* knob2) {
+inline int ring_balanced_grid(long long total, long long slots, int alone, int shared) {
     long long g = slots;
     const int conc = atvs_concurrency() < 8 ? atvs_concurrency() : 8;
-    int minplanes = alone + (shared - alone) * (conc - 1) / 7;
-    if (const char* e = getenv("ATVS_RING_MINPLANES")) minplanes = atoi(e) > 0 ? atoi(e) : minplanes;
+    const int minplanes = alone + (shared - alone) * (conc - 1) / 7;
     if (total / g < minplanes) g = total / minplanes;
     {   // small volumes: never fewer than 16 CTAs (of >= 6 planes) - a layer of 320 planes on 2 CTAs would serialise its pass
         long long floor_g = total / 6 < 16 ? total / 6 : 16;
         if (g < floor_g) g = floor_g;
     }
-    const char* e = knob1 ? getenv(knob1) : nullptr;
-    if (!e && knob2) e = getenv(knob2);
-    if (e && atoi(e) > 0) g = atoi(e) < slots ? atoi(e) : slots;
     if (g > total) g = total;
     if (g < 1) g = 1;
     return (int)g;
-}
-
-// z-segment length of a plane-ring kernel's work units.  A unit costs (planes + startup) plane steps, where `startup`
-// stands for the per-CTA fixed cost (TMEM allocation, weight image, pipeline fill) in plane steps.  The kernel shares
-// the GPU with the other passes of a depth map (4-8 streams), so it is charged as if a fraction `share` of the
-// `slots` (SMs x CTAs per SM) were its own; the real wave count bounds it from below.  Measured on the whole cfg2 step
-// (tools/tune_step.py, profiles/r02_tune_step.txt): per-kernel-optimal short units (many CTAs) cost 0.8 ms of 6.7.
-//   cols: tile columns, nz: planes along z, planes(zs) = per_z * zs + halo plane steps per unit
-inline int ring_pick_zs(long long cols, int nz, long long slots, int per_z, int halo, double share, double startup,
-                        int zmin) {
-    double best = -1.0;
-    int bz = nz;
-    const double mine = share * (double)slots;
-    for (int zs = (nz < zmin ? nz : zmin); zs <= nz; ++zs) {
-        const long long units = cols * ((nz + zs - 1) / zs);
-        double waves = (double)((units + slots - 1) / slots);
-        if ((double)units / mine > waves) waves = (double)units / mine;
-        const double cost = waves * ((double)(per_z * zs + halo) + startup);
-        if (best < 0.0 || cost < best - 1e-9) { best = cost; bz = zs; }
-    }
-    return bz;
 }
 
 }  // namespace

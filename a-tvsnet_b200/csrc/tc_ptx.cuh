@@ -31,31 +31,19 @@ __device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
 __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
-// ATVS_MBAR_HINT_NS: suspend-time hint of mbarrier.try_wait in ns; 0 = no hint (the hardware's default time limit).
-// Measured both ways (profiles/r02_ring_probe.txt): the kernels alone do not care, the whole cfg2 step is 0.08 ms faster
-// with the long hint (waiting warps sleep instead of polling while 8 streams share the SMs).
-#ifndef ATVS_MBAR_HINT_NS
-#define ATVS_MBAR_HINT_NS 10000000
-#endif
+// suspend-time hint of mbarrier.try_wait in ns.  Measured against no hint (the hardware's default time limit,
+// profiles/r02_ring_probe.txt): the kernels alone do not care, the whole cfg2 step is 0.08 ms faster with the long hint
+// (waiting warps sleep instead of polling while 8 streams share the SMs).
+constexpr uint32_t MBAR_HINT_NS = 10000000;
 __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
     uint32_t ok;
-#if ATVS_MBAR_HINT_NS > 0
     asm volatile(
         "{\n\t.reg .pred p;\n\t"
         "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\t"
         "selp.u32 %0, 1, 0, p;\n\t}"
         : "=r"(ok)
-        : "r"(smem_u32(bar)), "r"(parity), "r"((uint32_t)ATVS_MBAR_HINT_NS)
+        : "r"(smem_u32(bar)), "r"(parity), "r"(MBAR_HINT_NS)
         : "memory");
-#else
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-#endif
     return ok != 0;
 }
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {

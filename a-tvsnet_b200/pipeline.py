@@ -15,7 +15,7 @@ from .model import _prob2depth, build_cost_volume
 # tensor-core path: run the first CRM layers on the warped half only (network.SplitCostVolume)
 SPLIT_COST_VOLUME = True
 # number of CUDA streams the independent stage-I passes are spread over
-CONCURRENT_PASSES = int(__import__('os').environ.get('ATVS_PASSES', '8'))
+CONCURRENT_PASSES = 8
 
 
 def _cost_volume(r, v, cams, depth_num, depth_start, depth_interval, rid, vid, v16=None):

@@ -68,9 +68,10 @@ def test_argument_errors_without_gpu(lib):
     assert lib.atvs_visual_hull(p, p, p, p, p, 1, 4, 4, 4, 3, 1, p, None) == -5                        # view_num must be 2
     assert lib.atvs_refine_geo_group(p, p, p, p, p, p, p, 1, 4, 1, 4, 16, p, None) == -1               # H > 1
     assert lib.atvs_refine_photo_group(p, p, None, p, 1, 4, 4, 4, 16, p, None) == -4
-    # per-tap TMA image + halo-ring images (stride 1, and stride 2 for Cin <= 32)
+    # per-tap TMA image + halo-ring images (stride 1, and stride 2 for Cin <= 16)
     assert lib.atvs_packed_weight_bytes(64, 64, 0) == 2 * 27 * 2 * 32 * 64 + 2 * 36 * 2 * 96 * 16
     assert lib.atvs_packed_weight_bytes(8, 8, 0) == 28 * 16 * 8 * 2 + 5 * 2 * 64 * 16 + 5 * 2 * 48 * 16
+    assert lib.atvs_packed_weight_bytes(32, 16, 0) == 27 * 16 * 32 * 2 + 18 * 2 * 48 * 16
     # per-class image + fused 8-class image + plane-ring image [4 shifts][2 chunks][3 planes x 4 classes x 8][8]
     assert lib.atvs_packed_weight_bytes(16, 8, 1) == 27 * 16 * 16 * 2 * 2 + 4 * 2 * 96 * 16
 

@@ -15,9 +15,4 @@ ncu --set full --clock-control none --import-source on --profile-from-start off 
     -f -o /tmp/${TAG}_hot python tools/profile_step.py --views 2 > gpurun_out/${TAG}_ncu_f.log 2>&1
 python tools/ncu_summary.py /tmp/${TAG}_hot.ncu-rep > gpurun_out/${TAG}_ncu_full_hot_kernels_summary.txt
 python tools/ncu_traffic.py /tmp/${TAG}_hot.ncu-rep gpurun_out/${TAG}_ncu_traffic.json > gpurun_out/${TAG}_ncu_traffic.txt
-# K2 (one-kernel attention aggregation) at cfg2 size, 4 views: one full capture of the kernel itself
-ncu --set full --clock-control none --import-source on -k regex:'k_attention_ring' -c 1 \
-    -f -o /tmp/${TAG}_attn python tools/attn_probe.py > gpurun_out/${TAG}_ncu_a.log 2>&1
-python tools/ncu_summary.py /tmp/${TAG}_attn.ncu-rep > gpurun_out/${TAG}_ncu_full_k2_summary.txt
-python tools/ncu_traffic.py /tmp/${TAG}_attn.ncu-rep gpurun_out/${TAG}_ncu_k2_traffic.json > gpurun_out/${TAG}_ncu_k2_traffic.txt
 ls -la gpurun_out/${TAG}_*
