@@ -46,12 +46,14 @@ def stage1_forward(features, cams, depth_num, depth_start, depth_interval, view_
     return tower.get_output_by_name('conv_b2_6_1'), tower.get_output().squeeze(-1)
 
 
-def stage1_reverse(features, cams, depth_num, depth_start, depth_interval, view_i, features16=None):
-    """reverse half (model.py:413-415): view_i as reference -> depth_view (B,h,w,1)."""
+def stage1_reverse(features, cams, depth_num, depth_start, depth_interval, view_i, features16=None, confidence=False):
+    """reverse half (model.py:413-415): view_i as reference -> depth_view (B,h,w,1); with ``confidence`` the pair
+    (depth_view, its probability map (B,h,w,1)), both from the same soft-argmin launch."""
     cvv = _cost_volume(features[:, view_i], features[:, 0], cams, depth_num, depth_start, depth_interval, view_i, 0,
                        None if features16 is None else features16[:, 0])
     pv = StackedUNet_prob({'data': cvv}, outputs=('conv_b2_6_2',)).get_output().squeeze(-1)
-    return _prob2depth(pv, depth_start, depth_interval, 1, False)[0]
+    depth_view, prob_map = _prob2depth(pv, depth_start, depth_interval, 1, confidence)
+    return (depth_view, prob_map) if confidence else depth_view
 
 
 def stage1_view(features, cams, depth_num, depth_start, depth_interval, view_i, siamese=True):
@@ -156,9 +158,12 @@ def shard_views(n_views, rank, world):
     return [v for v in range(1, n_views) if (v - 1) % world == rank]
 
 
-def run_multiview(features, cams, depth_num, siamese=True, upsample=True, group=None, rank=0, world=1):
+def run_multiview(features, cams, depth_num, siamese=True, upsample=True, group=None, rank=0, world=1, confidence=False):
     """features (B,N,h,w,F) fp32, cams (B,N,2,4,4) -> dict(depth (B,h,w,1), depth_up (B,4h,4w,1),
-    prob_volume_agg, cost_volume_agg, depth_views).  example.py:144-158 + :109 (x4 upsample)."""
+    prob_volume_agg, cost_volume_agg, depth_views).  example.py:144-158 + :109 (x4 upsample).
+    ``confidence`` adds the probability maps of prob2depth_upsample(out_prob_map=True) (model.py:113-129, :13-65),
+    each from the soft-argmin launch of its depth map: prob_map (B,h,w,1), prob_map_up (B,4h,4w,1) with ``upsample``,
+    and depth_view_probs beside depth_views (None entries without ``siamese``)."""
     L.require_cuda(features, cams)
     cams = L.f32c(cams)
     n_views = cams.shape[1]
@@ -185,7 +190,7 @@ def run_multiview(features, cams, depth_num, siamese=True, upsample=True, group=
 
     def run_task(v, kind):
         if kind == 'r':
-            return stage1_reverse(features, cams, depth_num, ds, di, v, feats16)
+            return stage1_reverse(features, cams, depth_num, ds, di, v, feats16, confidence)
         out = stage1_forward(features, cams, depth_num, ds, di, v, feats16)
         if att_raw is not None:
             N.attention_raw_view(att_raw, mine.index(v), N.to_act(out[0]), 'attention_aggregate')
@@ -217,29 +222,36 @@ def run_multiview(features, cams, depth_num, siamese=True, upsample=True, group=
             main.wait_stream(st)
     L.call("atvs_set_concurrency", 1)      # stage II runs alone on the calling stream
     filtered = [results[(v, 'f')][0] for v in mine]
-    depth_views = [results[(v, 'r')] for v in mine] if siamese else [None for _ in mine]
+    reverse = [results[(v, 'r')] if siamese else None for v in mine]
+    depth_views = [r[0] if confidence and r is not None else r for r in reverse]
     cost_agg = aggregate(filtered, 'attention_aggregate', group, rank, world, raw=att_raw)
     prob_agg = OutputConv({'data': cost_agg}).get_output().squeeze(-1)
-    depth, _ = _prob2depth(prob_agg, ds, di, 1, False)
+    depth, prob_map = _prob2depth(prob_agg, ds, di, 1, confidence)
     out = dict(depth=depth, prob_volume_agg=prob_agg, cost_volume_agg=cost_agg, depth_views=depth_views)
+    if confidence:
+        out.update(prob_map=prob_map, depth_view_probs=[None if r is None else r[1] for r in reverse])
     if upsample:
-        out['depth_up'], _ = _prob2depth(prob_agg, ds, di, 4, False)
+        out['depth_up'], prob_map_up = _prob2depth(prob_agg, ds, di, 4, confidence)
+        if confidence:
+            out['prob_map_up'] = prob_map_up
     return out
 
 
-def run_example_schedule(images, cams, depth_num, features=None):
+def run_example_schedule(images, cams, depth_num, features=None, confidence=False):
     """The whole four-stage schedule of example.py:144-181 on the device, images in:
       I   per source view: FEM features -> TVSNet_base_siamese -> (filtered cost, prob volume, depth_view)
       II  AAM1 (keepchannel) -> output_conv -> prob2depth                              (run_multiview)
       III per source view: TVSNet_refine(depth_agg_init, depth_view_n, prob_agg, cost_agg, images, cams)   (refine.py, fp32)
       IV  AAM2 (keepchannel) -> output_conv_refine -> prob2depth_upsample -> final x4 inverse-depth map
-    images (B,N,H,W,3) fp32 0..255, cams (B,N,2,4,4) at feature resolution.  ``features`` (B,N,h,w,32) skips the FEM."""
+    images (B,N,H,W,3) fp32 0..255, cams (B,N,2,4,4) at feature resolution.  ``features`` (B,N,h,w,32) skips the FEM.
+    ``confidence`` adds the stage-II keys of run_multiview(confidence=True) and the stage-IV probability maps
+    refined_prob_map (B,h,w,1) and refined_prob_map_up (B,4h,4w,1)."""
     from . import fem, refine
     from .atvsnet import OutputConv_refine
     L.require_cuda(images, cams)
     cams = L.f32c(cams)
     feats = features if features is not None else fem.extract_features(images)
-    out = run_multiview(feats, cams, depth_num, siamese=True, upsample=False)
+    out = run_multiview(feats, cams, depth_num, siamese=True, upsample=False, confidence=confidence)
     ds = cams[:, 0, 1, 3, 0].contiguous()
     di = cams[:, 0, 1, 3, 1].contiguous()
     n_views = cams.shape[1]
@@ -253,25 +265,31 @@ def run_example_schedule(images, cams, depth_num, features=None):
             refined_costs.append(rc)
     cost_ref = N.attention_aggregation(refined_costs, 'attention_aggregate_refine')
     prob_ref = OutputConv_refine({'data': cost_ref}).get_output().squeeze(-1)
-    out['depth_refined'], _ = _prob2depth(prob_ref, ds, di, 1, False)
-    out['depth_refined_up'], _ = _prob2depth(prob_ref, ds, di, 4, False)
+    out['depth_refined'], pm = _prob2depth(prob_ref, ds, di, 1, confidence)
+    out['depth_refined_up'], pm_up = _prob2depth(prob_ref, ds, di, 4, confidence)
     out.update(refined_cost_volume_agg=cost_ref, refined_prob_volume_agg=prob_ref, refined_prob_volumes=refined_probs)
+    if confidence:
+        out.update(refined_prob_map=pm, refined_prob_map_up=pm_up)
     return out
 
 
-def run_twoview(images, cams, depth_num):
+def run_twoview(images, cams, depth_num, confidence=False):
     """The two-view driver of example.py:219-272 (run_test_twoview; taken when only two views exist, example.py:344-347):
     TVSNet (FEM on both images, both directions, refinement) -> prob2depth_upsample.  images (B,2,H,W,3) raw 0..255 BGR,
-    cams (B,2,2,4,4) at feature resolution -> dict(refined_prob_volume, depth_refined, depth_refined_up)."""
+    cams (B,2,2,4,4) at feature resolution -> dict(refined_prob_volume, depth_refined, depth_refined_up), with
+    ``confidence`` also refined_prob_map (B,h,w,1) and refined_prob_map_up (B,4h,4w,1)."""
     from .model import TVSNet
     L.require_cuda(images, cams)
     cams = L.f32c(cams)
     ds = cams[:, 0, 1, 3, 0].contiguous()
     di = cams[:, 0, 1, 3, 1].contiguous()
     refined = TVSNet(images, cams, depth_num, ds, di, view_i=1, ref_i=0)
-    est, _ = _prob2depth(refined, ds, di, 1, False)
-    est_up, _ = _prob2depth(refined, ds, di, 4, False)
-    return dict(refined_prob_volume=refined, depth_refined=est, depth_refined_up=est_up)
+    est, pm = _prob2depth(refined, ds, di, 1, confidence)
+    est_up, pm_up = _prob2depth(refined, ds, di, 4, confidence)
+    out = dict(refined_prob_volume=refined, depth_refined=est, depth_refined_up=est_up)
+    if confidence:
+        out.update(refined_prob_map=pm, refined_prob_map_up=pm_up)
+    return out
 
 
 def inverse_to_depth(out, twoview=False):
@@ -282,18 +300,20 @@ def inverse_to_depth(out, twoview=False):
     return 1.0 / out
 
 
-def run_example(images, cams, depth_num=None):
+def run_example(images, cams, depth_num=None, confidence=False):
     """example.py:main dispatch (:344-347): the multi-view schedule for more than two views, the two-view network
-    otherwise.  Returns the final x4 inverse-depth map (B,H,W,1) and ``pred`` = depth (what example.py saves)."""
+    otherwise.  Returns the final x4 inverse-depth map (B,H,W,1) and ``pred`` = depth (what example.py saves); with
+    ``confidence`` also ``prob`` = the x4 probability map of that final depth map (refined_prob_map_up)."""
     n_views = cams.shape[1]
     D = int(depth_num if depth_num is not None else N.FLAGS.max_d)
     if n_views > 2:
-        out = run_example_schedule(images, cams, D)
-        inv = out['depth_refined_up']
+        out = run_example_schedule(images, cams, D, confidence=confidence)
     else:
-        out = run_twoview(images, cams, D)
-        inv = out['depth_refined_up']
+        out = run_twoview(images, cams, D, confidence=confidence)
+    inv = out['depth_refined_up']
     out['pred'] = inverse_to_depth(inv, twoview=n_views <= 2)
+    if confidence:
+        out['prob'] = out['refined_prob_map_up']
     if N.act_dtype() in N.HALF_DTYPES:
         check_saturation()
     return out
@@ -329,9 +349,12 @@ class FrameStream(object):
         fs = FrameStream(feats_shape, cams_shape, depth_num, device)
         for depth_h in fs.run(frames):      # frames: iterable of (feats_pinned, cams_pinned)
             ...                              # depth_h: pinned (B,4h,4w,1) fp32, valid until two frames later
+
+    With ``confidence=True`` the graph also computes the x4 probability map (run_multiview's prob_map_up) and ``run``
+    yields pinned (depth_h, confidence_h) pairs of that shape, copied and kept valid like the depth map alone.
     """
 
-    def __init__(self, feats_shape, cams_shape, depth_num, device, siamese=True):
+    def __init__(self, feats_shape, cams_shape, depth_num, device, siamese=True, confidence=False):
         self.device = torch.device(device)
         self.depth_num = int(depth_num)
         dev = self.device
@@ -341,25 +364,32 @@ class FrameStream(object):
         self.stage_c = [torch.empty_like(self.cams) for _ in range(2)]
         self.s_in, self.s_out = torch.cuda.Stream(device=dev), torch.cuda.Stream(device=dev)
         self.siamese = siamese
+        self.confidence = confidence
         self.graph = None
         self.out = None
 
+    def _step(self):
+        return run_multiview(self.feats, self.cams, self.depth_num, siamese=self.siamese, confidence=self.confidence)
+
     def _capture(self):
         for _ in range(3):      # eager warm-up: packs the weights, sets kernel attributes, fills the allocator
-            run_multiview(self.feats, self.cams, self.depth_num, siamese=self.siamese)
+            self._step()
         torch.cuda.synchronize(self.device)
         s = torch.cuda.Stream(device=self.device)
         s.wait_stream(torch.cuda.current_stream(self.device))
         with torch.cuda.stream(s):
             self.graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(self.graph, stream=s):
-                self.out = run_multiview(self.feats, self.cams, self.depth_num, siamese=self.siamese)['depth_up']
+                res = self._step()
+                self.out = [res[k] for k in (('depth_up', 'prob_map_up') if self.confidence else ('depth_up',))]
         torch.cuda.current_stream(self.device).wait_stream(s)
-        self.stage_o = [torch.empty_like(self.out) for _ in range(2)]
-        self.host_o = [torch.empty(self.out.shape, dtype=torch.float32).pin_memory() for _ in range(2)]
+        # per output: staging slot k on the device and its pinned host copy, k = frame index & 1
+        self.stage_o = [[torch.empty_like(o) for o in self.out] for _ in range(2)]
+        self.host_o = [[torch.empty(o.shape, dtype=torch.float32).pin_memory() for o in self.out] for _ in range(2)]
 
     def run(self, frames):
-        """generator over pinned host depth maps, one per frame, in order (each is yielded once its copy is complete)."""
+        """generator over pinned host depth maps, one per frame, in order (each is yielded once its copy is complete);
+        (depth, confidence) pairs with ``confidence=True``."""
         main = torch.cuda.current_stream(self.device)
         first = True
         free = [None, None]          # staging slot reusable once the step that read it has copied it out
@@ -389,15 +419,17 @@ class FrameStream(object):
             self.graph.replay()
             if done[k] is not None:
                 main.wait_event(done[k])          # stage_o[k] / host_o[k] of frame i-2 have been drained
-            self.stage_o[k].copy_(self.out, non_blocking=True)
+            for so, o in zip(self.stage_o[k], self.out):
+                so.copy_(o, non_blocking=True)
             computed = torch.cuda.Event()
             computed.record(main)
             with torch.cuda.stream(self.s_out):
                 self.s_out.wait_event(computed)
-                self.host_o[k].copy_(self.stage_o[k], non_blocking=True)
+                for ho, so in zip(self.host_o[k], self.stage_o[k]):
+                    ho.copy_(so, non_blocking=True)
                 done[k] = torch.cuda.Event()
                 done[k].record(self.s_out)
-            pending.append((done[k], self.host_o[k]))
+            pending.append((done[k], tuple(self.host_o[k]) if self.confidence else self.host_o[k][0]))
             if len(pending) > 1:
                 ev, buf = pending.pop(0)
                 ev.synchronize()
