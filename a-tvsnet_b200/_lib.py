@@ -1,6 +1,7 @@
 """ctypes binding of libatvs.so (include/atvs.h).  There is NO fallback: if the library
 is missing or a call fails, a RuntimeError is raised."""
 import ctypes as C
+import functools
 import os
 
 import torch
@@ -101,6 +102,45 @@ def ptr(t):
 
 def stream():
     return C.c_void_p(torch.cuda.current_stream().cuda_stream)
+
+
+def _cuda_devices(obj, found):
+    if isinstance(obj, torch.Tensor):
+        if obj.is_cuda:
+            found.add(obj.device.index)
+    elif isinstance(obj, (list, tuple)):
+        for o in obj:
+            _cuda_devices(o, found)
+    elif isinstance(obj, dict):
+        for o in obj.values():
+            _cuda_devices(o, found)
+    else:      # e.g. network.SplitCostVolume
+        d = getattr(obj, 'device', None)
+        if isinstance(d, torch.device) and d.type == 'cuda':
+            found.add(d.index)
+
+
+def input_device(args, who='a-tvsnet_b200'):
+    """``with input_device(args):`` makes the device of the CUDA tensors in ``args`` (tensors, lists, tuples, dicts,
+    objects with a ``.device``) the current one, so that every launch goes to that device's current stream and the
+    variable store hands out that device's weights (variables.get_variable), and restores the caller's current device
+    on exit.  CUDA tensors on different devices raise ValueError before anything is launched; without CUDA tensors
+    the current device stays."""
+    found = set()
+    _cuda_devices(args, found)
+    if len(found) > 1:
+        raise ValueError("%s: CUDA inputs on different devices (%s); move them to one device"
+                         % (who, ', '.join('cuda:%d' % i for i in sorted(found))))
+    return torch.cuda.device(found.pop() if found else -1)
+
+
+def on_input_device(fn):
+    """decorator of a public entry point: the call runs under input_device(its arguments)."""
+    @functools.wraps(fn)
+    def entry(*args, **kwargs):
+        with input_device((args, kwargs), fn.__name__):
+            return fn(*args, **kwargs)
+    return entry
 
 
 def require_cuda(*tensors):

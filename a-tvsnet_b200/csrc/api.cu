@@ -1,7 +1,6 @@
 // api.cu - version / error string / device query of the C ABI (include/atvs.h).
 #include "common.cuh"
 #include <stdarg.h>
-#include <atomic>
 
 static thread_local char g_err[512] = "";
 
@@ -49,19 +48,45 @@ static std::atomic<long long> g_launches{0};
 void atvs_count_launch() { g_launches.fetch_add(1, std::memory_order_relaxed); }
 extern "C" long long atvs_launch_count(void) { return g_launches.load(std::memory_order_relaxed); }
 
-// how many independent passes the caller runs side by side on its streams (pipeline.run_multiview): the plane-ring
-// kernels size their grids with it (ring_common.cuh ring_balanced_grid)
-static std::atomic<int> g_concurrency{1};
-int atvs_concurrency() { return g_concurrency.load(std::memory_order_relaxed); }
-extern "C" int atvs_set_concurrency(int n) {
-    g_concurrency.store(n < 1 ? 1 : (n > 64 ? 64 : n), std::memory_order_relaxed);
+int atvs_current_device(int* dev) {
+    ATVS_CUDA(cudaGetDevice(dev));
+    ATVS_CHECK_ARG(*dev >= 0 && *dev < ATVS_MAX_DEVICES, ATVS_E_UNSUP, "device %d: the library keeps state for devices "
+                   "0..%d", *dev, ATVS_MAX_DEVICES - 1);
     return 0;
 }
 
-static unsigned long long* g_sat[64] = {nullptr};
+static std::atomic<int> g_sms[ATVS_MAX_DEVICES];
+int atvs_num_sms() {
+    int dev = 0;
+    if (atvs_current_device(&dev) != 0) return 148;
+    int n = g_sms[dev].load(std::memory_order_relaxed);
+    if (n == 0) {
+        if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0) n = 148;
+        g_sms[dev].store(n, std::memory_order_relaxed);
+    }
+    return n;
+}
+
+// per device: how many independent passes the caller runs side by side on its streams (pipeline.run_multiview); the
+// plane-ring kernels size their grids with it (ring_common.cuh ring_balanced_grid).  0 = never set = 1.
+static std::atomic<int> g_concurrency[ATVS_MAX_DEVICES];
+int atvs_concurrency() {
+    int dev = 0;
+    if (atvs_current_device(&dev) != 0) return 1;
+    const int n = g_concurrency[dev].load(std::memory_order_relaxed);
+    return n < 1 ? 1 : n;
+}
+extern "C" int atvs_set_concurrency(int n) {
+    int dev = 0;
+    if (const int rc = atvs_current_device(&dev)) return rc;
+    g_concurrency[dev].store(n < 1 ? 1 : (n > 64 ? 64 : n), std::memory_order_relaxed);
+    return 0;
+}
+
+static unsigned long long* g_sat[ATVS_MAX_DEVICES] = {nullptr};
 unsigned long long* atvs_sat_ptr() {
     int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return nullptr;
+    if (atvs_current_device(&dev) != 0) return nullptr;
     if (g_sat[dev] == nullptr) {
         unsigned long long* p = nullptr;
         if (cudaMalloc(&p, sizeof(unsigned long long)) != cudaSuccess) { cudaGetLastError(); return nullptr; }

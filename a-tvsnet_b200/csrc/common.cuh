@@ -5,6 +5,7 @@
 #include <cuda_fp16.h>
 #include <stdint.h>
 #include <stdio.h>
+#include <atomic>
 #include "../../include/atvs.h"
 
 void atvs_set_error(const char* fmt, ...);
@@ -31,19 +32,30 @@ void atvs_count_launch();
 // device counter (one per device, allocated on first use - never during stream capture: every path is warmed up
 // eagerly first) of fp16 raw-output rows that had to be clamped to +-65504; read with atvs_saturation_count()
 unsigned long long* atvs_sat_ptr();
-int atvs_concurrency();          // api.cu: passes the caller runs side by side (atvs_set_concurrency)
+int atvs_concurrency();          // api.cu: passes the caller runs side by side on the current device
 #define ATVS_LAUNCH_CHECK()              \
     do {                                 \
         atvs_count_launch();             \
         ATVS_CUDA(cudaPeekAtLastError()); \
     } while (0)
 
-static inline int atvs_num_sms() {
-    static int n = 0;
-    if (n == 0) {
-        int dev = 0;
-        if (cudaGetDevice(&dev) != cudaSuccess) return 148;
-        if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0) n = 148;
+// State the library keeps per device (include/atvs.h) is indexed by the device ordinal.
+#define ATVS_MAX_DEVICES 64
+// *dev = the calling thread's current device, which every launch and query of the library applies to; 0, or the
+// failing call's code with the message set (also for an ordinal beyond ATVS_MAX_DEVICES)
+int atvs_current_device(int* dev);
+int atvs_num_sms();              // api.cu: SMs of the current device (148 when it cannot be read)
+
+// Opts KERNEL in to 227 KB of dynamic shared memory.  A function attribute belongs to the device that was current
+// when it was set, so it is set once per (kernel, device); threads that race on a first launch set the same value.
+template <auto KERNEL>
+int atvs_max_dynamic_smem() {
+    static std::atomic<bool> done[ATVS_MAX_DEVICES];
+    int dev = 0;
+    if (const int rc = atvs_current_device(&dev)) return rc;
+    if (!done[dev].load(std::memory_order_acquire)) {
+        ATVS_CUDA(cudaFuncSetAttribute(KERNEL, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+        done[dev].store(true, std::memory_order_release);
     }
-    return n;
+    return 0;
 }

@@ -377,12 +377,7 @@ k_attention_ring(const __grid_constant__ AttnParams p, const uint8_t* __restrict
 
 template <int NMAX, int G, int MINB, bool F16>
 int launch_attn(const AttnParams& p, const uint8_t* wimg, float* out, size_t smem, int grid, cudaStream_t st) {
-    static bool attr_set = false;
-    if (!attr_set) {
-        ATVS_CUDA(cudaFuncSetAttribute(k_attention_ring<NMAX, G, MINB, F16>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       227 * 1024));
-        attr_set = true;
-    }
+    if (const int rc = atvs_max_dynamic_smem<k_attention_ring<NMAX, G, MINB, F16>>()) return rc;
     k_attention_ring<NMAX, G, MINB, F16><<<grid, AR_THREADS, smem, st>>>(p, wimg, out);
     ATVS_LAUNCH_CHECK();
     return 0;

@@ -261,11 +261,7 @@ __global__ void k_pack_deconv(const float* __restrict__ w, int Cin, int Cout, in
 
 template <int CIN, int NPAD>
 int launch_dc(const DcMaps& maps, const DcParams& p, float* out, double* stats, size_t smem, int grid, cudaStream_t st) {
-    static bool attr_set = false;
-    if (!attr_set) {
-        ATVS_CUDA(cudaFuncSetAttribute(k_deconv3d_tc<CIN, NPAD>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        attr_set = true;
-    }
+    if (const int rc = atvs_max_dynamic_smem<k_deconv3d_tc<CIN, NPAD>>()) return rc;
     k_deconv3d_tc<CIN, NPAD><<<grid, DC_THREADS, smem, st>>>(maps, p, out, stats);
     ATVS_LAUNCH_CHECK();
     return 0;

@@ -377,11 +377,7 @@ __global__ void k_pack_deconv_ring(const float* __restrict__ w, int Cin, int Cou
 template <int CIN, int COUT>
 int launch_dr(const uint16_t* x, const DrParams& p, const uint8_t* wimg, float* out, double* stats, size_t smem, int grid,
               cudaStream_t st) {
-    static bool attr_set = false;
-    if (!attr_set) {
-        ATVS_CUDA(cudaFuncSetAttribute(k_deconv3d_ring<CIN, COUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        attr_set = true;
-    }
+    if (const int rc = atvs_max_dynamic_smem<k_deconv3d_ring<CIN, COUT>>()) return rc;
     k_deconv3d_ring<CIN, COUT><<<grid, DR_THREADS, smem, st>>>(x, p, wimg, out, stats);
     ATVS_LAUNCH_CHECK();
     return 0;

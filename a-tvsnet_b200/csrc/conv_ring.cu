@@ -545,11 +545,7 @@ __global__ void k_pack_ring(const float* __restrict__ w, int Cin, int Cout, int 
 template <int CIN, int CP, int MINB, bool FAST>
 int launch_ring1(const uint16_t* x, const RingParams& p, const uint8_t* wimg, float* out, double* stats,
                  const float* bias, size_t smem, int grid, cudaStream_t st) {
-    static bool attr_set = false;
-    if (!attr_set) {
-        ATVS_CUDA(cudaFuncSetAttribute(k_conv3d_ring<CIN, CP, MINB, FAST>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        attr_set = true;
-    }
+    if (const int rc = atvs_max_dynamic_smem<k_conv3d_ring<CIN, CP, MINB, FAST>>()) return rc;
     k_conv3d_ring<CIN, CP, MINB, FAST><<<grid, RG_THREADS, smem, st>>>(x, p, wimg, out, stats, bias);
     ATVS_LAUNCH_CHECK();
     return 0;

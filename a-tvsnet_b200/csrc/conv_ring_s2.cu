@@ -391,11 +391,7 @@ __global__ void k_pack_ring_s2(const float* __restrict__ w, int Cin, int Cout, i
 template <int CIN, int CP, int MINB>
 int launch_s2(const uint16_t* x, const S2Params& p, const uint8_t* wimg, float* out, double* stats,
               const float* bias, size_t smem, int grid, cudaStream_t st) {
-    static bool attr_set = false;
-    if (!attr_set) {
-        ATVS_CUDA(cudaFuncSetAttribute(k_conv3d_ring_s2<CIN, CP, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        attr_set = true;
-    }
+    if (const int rc = atvs_max_dynamic_smem<k_conv3d_ring_s2<CIN, CP, MINB>>()) return rc;
     k_conv3d_ring_s2<CIN, CP, MINB><<<grid, S2_THREADS, smem, st>>>(x, p, wimg, out, stats, bias);
     ATVS_LAUNCH_CHECK();
     return 0;

@@ -311,11 +311,7 @@ int ntaps_padded(int Cin, int transposed, int cls) {
 template <int CIN, int NPAD>
 int launch_tc(const TcMaps& maps, const TcParams& p, float* out, double* stats, const float* bias, size_t smem,
               int grid, cudaStream_t st) {
-    static bool attr_set = false;
-    if (!attr_set) {
-        ATVS_CUDA(cudaFuncSetAttribute(k_conv3d_tc<CIN, NPAD>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        attr_set = true;
-    }
+    if (const int rc = atvs_max_dynamic_smem<k_conv3d_tc<CIN, NPAD>>()) return rc;
     k_conv3d_tc<CIN, NPAD><<<grid, TC_THREADS, smem, st>>>(maps, p, out, stats, bias);
     ATVS_LAUNCH_CHECK();
     return 0;

@@ -625,19 +625,19 @@ extern "C" int atvs_conv3d_fp32(const float* x, const float* kernel, int B, int 
     return 0;
 }
 
-// grid of a grid-stride kernel = exactly the blocks that are resident at once (occupancy API, cached per kernel): a
-// grid of 8 blocks per SM with 6 resident runs as 1.33 waves and idles a third of the machine in the second one
-template <typename K>
-static unsigned grid_resident(K kernel, long long n, int block) {
-    static int per_sm = 0;          // one instance per kernel type K ... and per kernel pointer below
-    static K cached = nullptr;
-    if (cached != kernel || per_sm == 0) {
-        int b = 0;
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, kernel, block, 0) != cudaSuccess || b < 1) b = 4;
-        per_sm = b;
-        cached = kernel;
+// grid of a grid-stride kernel = exactly the blocks that are resident at once (occupancy API, cached per kernel and
+// device): a grid of 8 blocks per SM with 6 resident runs as 1.33 waves and idles a third of the machine in the second one
+template <auto KERNEL>
+static unsigned grid_resident(long long n, int block) {
+    static std::atomic<int> per_sm[ATVS_MAX_DEVICES];       // 0 = not queried yet on that device
+    int dev = 0;
+    if (atvs_current_device(&dev) != 0) return grid_for(n, block, 4);
+    int b = per_sm[dev].load(std::memory_order_relaxed);
+    if (b == 0) {
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, KERNEL, block, 0) != cudaSuccess || b < 1) b = 4;
+        per_sm[dev].store(b, std::memory_order_relaxed);
     }
-    return grid_for(n, block, per_sm);
+    return grid_for(n, block, b);
 }
 
 template <typename RawT>
@@ -645,16 +645,16 @@ static int bn_relu_add_launch(const RawT* raw, const double* stats, const RawT* 
                               int C, float eps, int relu, const void* skip1, const void* skip2, void* out_plain,
                               void* out_sum, int act_dtype, cudaStream_t st, const char* who) {
     if (act_dtype == ATVS_F32) {
-        const unsigned grid = grid_resident(k_bn_relu_add<float, RawT>, count * C / 8 + 1, 256);
+        const unsigned grid = grid_resident<k_bn_relu_add<float, RawT>>(count * C / 8 + 1, 256);
         k_bn_relu_add<float, RawT><<<grid, 256, 0, st>>>(raw, stats, raw2, stats2, count, C, eps, relu, (const float*)skip1,
                                                          (const float*)skip2, (float*)out_plain, (float*)out_sum);
     } else if (act_dtype == ATVS_BF16) {
-        const unsigned grid = grid_resident(k_bn_relu_add<__nv_bfloat16, RawT>, count * C / 8 + 1, 256);
+        const unsigned grid = grid_resident<k_bn_relu_add<__nv_bfloat16, RawT>>(count * C / 8 + 1, 256);
         k_bn_relu_add<__nv_bfloat16, RawT><<<grid, 256, 0, st>>>(raw, stats, raw2, stats2, count, C, eps, relu,
                                                                  (const __nv_bfloat16*)skip1, (const __nv_bfloat16*)skip2,
                                                                  (__nv_bfloat16*)out_plain, (__nv_bfloat16*)out_sum);
     } else if (act_dtype == ATVS_F16) {
-        const unsigned grid = grid_resident(k_bn_relu_add<__half, RawT>, count * C / 8 + 1, 256);
+        const unsigned grid = grid_resident<k_bn_relu_add<__half, RawT>>(count * C / 8 + 1, 256);
         k_bn_relu_add<__half, RawT><<<grid, 256, 0, st>>>(raw, stats, raw2, stats2, count, C, eps, relu, (const __half*)skip1,
                                                           (const __half*)skip2, (__half*)out_plain, (__half*)out_sum);
     } else {
@@ -834,10 +834,10 @@ extern "C" int atvs_attention_raw(const void* act_raw, int act_dtype, const void
 #define ATT_RAW_N(T, M, NM)                                                                                   \
     do {                                                                                                      \
         if (act_dtype == ATVS_F16)                                                                            \
-            k_attention_raw<T, __half, M, NM><<<grid_resident(k_attention_raw<T, __half, M, NM>, V * (C / 8), 256), 256, 0, st>>>( \
+            k_attention_raw<T, __half, M, NM><<<grid_resident<k_attention_raw<T, __half, M, NM>>(V * (C / 8), 256), 256, 0, st>>>( \
                 (const __half*)act_raw, xs, N, V, C, gmax, out);                                               \
         else                                                                                                  \
-            k_attention_raw<T, float, M, NM><<<grid_resident(k_attention_raw<T, float, M, NM>, V * (C / 8), 256), 256, 0, st>>>(   \
+            k_attention_raw<T, float, M, NM><<<grid_resident<k_attention_raw<T, float, M, NM>>(V * (C / 8), 256), 256, 0, st>>>(   \
                 (const float*)act_raw, xs, N, V, C, gmax, out);                                                \
     } while (0)
     // the per-view logits live in registers: instantiate for the view count (4 sources at cfg2) so that the

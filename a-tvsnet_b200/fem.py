@@ -37,6 +37,7 @@ def tc_supported(x, kernel, stride, explicit_pad):
             and cin <= 320 and cout <= 256 and x.shape[1] * x.shape[2] >= 128)
 
 
+@L.on_input_device
 def conv2d_tc(x, kernel, rate=1, bias=None, relu=False, out_dtype=torch.float32, stats=None):
     """stride-1 'SAME' convolution on the tensor cores: x (B,H,W,Cin) fp16 -> (B,H,W,Cout) fp32 | fp16
     = [relu](conv + bias); ``stats`` (2*Cout fp64, zeroed) receives the per-channel moments (conv_bn layers)."""
@@ -48,6 +49,7 @@ def conv2d_tc(x, kernel, rate=1, bias=None, relu=False, out_dtype=torch.float32,
     return out
 
 
+@L.on_input_device
 def to_half(x):
     if x.dtype == torch.float16:
         return x
@@ -62,6 +64,7 @@ def _same_pad(n, k_eff, s):
     return total // 2, out
 
 
+@L.on_input_device
 def conv2d(x, kernel, stride=1, rate=1, bias=None, relu=False, padding='SAME', explicit_pad=None):
     """x (B,H,W,Cin) fp32 cuda, kernel [k,k,Cin,Cout].  padding 'SAME' (TF) or 'VALID' after ``explicit_pad`` =
     (begin, end) zero rows/cols on both axes (the bottleneck's tf.pad + VALID, network.py:589-595)."""
@@ -96,6 +99,7 @@ BATCH_VIEWS = True       # extract_features: one batch over the views (fp32 path
 _GROUPS = 1
 
 
+@L.on_input_device
 def batch_norm(x, beta=None, relu=False, stats=None, out_dtype=torch.float32):
     """batch statistics over (B,H,W), biased variance, eps 1e-3, optional ``+ beta``, optional ReLU.  ``stats``: moments
     already accumulated by the producing convolution's epilogue; ``out_dtype`` fp16 feeds a tensor-core convolution.
@@ -125,6 +129,7 @@ def batch_norm(x, beta=None, relu=False, stats=None, out_dtype=torch.float32):
     return out
 
 
+@L.on_input_device
 def conv_bn(x, name, stride=1, rate=1, out_dtype=torch.float32):
     """network.py:173-215 on a 4-D tensor: name/conv2d/kernel, BN without affine, ReLU."""
     kernel = V.get_variable(name + '/conv2d/kernel')
@@ -135,6 +140,7 @@ def conv_bn(x, name, stride=1, rate=1, out_dtype=torch.float32):
     return batch_norm(conv2d(x, kernel, stride, rate), None, True, out_dtype=out_dtype)
 
 
+@L.on_input_device
 def add(a, b):
     if tuple(a.shape) != tuple(b.shape) or a.dtype != torch.float32 or b.dtype != torch.float32:
         raise ValueError("add: operands must be fp32 tensors of one shape, got %s %s and %s %s"
@@ -145,6 +151,7 @@ def add(a, b):
     return out
 
 
+@L.on_input_device
 def bottleneck(x, scope, depth, stride=1, rate=1):
     """network.py:552-603."""
     g = V.get_variable
@@ -175,6 +182,7 @@ def bottleneck(x, scope, depth, stride=1, rate=1):
     return add(shortcut, r)
 
 
+@L.on_input_device
 def res_block(x, name, depth, num_block, stride=1, rate=1):
     """network.py:605-616."""
     if num_block == 1:
@@ -185,6 +193,7 @@ def res_block(x, name, depth, num_block, stride=1, rate=1):
     return out
 
 
+@L.on_input_device
 def avg_pool(x, k, s):
     B, H, W, C = x.shape
     out = torch.empty((B, -(-H // s), -(-W // s), C), dtype=torch.float32, device=x.device)
@@ -192,6 +201,7 @@ def avg_pool(x, k, s):
     return out
 
 
+@L.on_input_device
 def image_resize(x, Ho, Wo):
     B, H, W, C = x.shape
     out = torch.empty((B, Ho, Wo, C), dtype=torch.float32, device=x.device)
@@ -199,6 +209,7 @@ def image_resize(x, Ho, Wo):
     return out
 
 
+@L.on_input_device
 def ResNetDS2SPP(image, return_layers=False):
     """cnn_wrapper/atvsnet.py:254-292: image (B,H,W,3) fp32 cuda -> feature (B,H/4,W/4,32) fp32."""
     L.require_cuda(image)
@@ -222,6 +233,7 @@ def ResNetDS2SPP(image, return_layers=False):
     return (out, layers) if return_layers else out
 
 
+@L.on_input_device
 def extract_features(images):
     """model.py:420-425 TVSNet_feature_extraction over all views: images (B,N,H,W,3) -> features (B,N,H/4,W/4,32).
     One tower per VIEW on the (B,H,W,3) slice, as in the reference: batch statistics are taken over the whole batch B

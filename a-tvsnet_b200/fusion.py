@@ -31,6 +31,7 @@ def cameras_from_krt(K, R, t):
     return tuple(torch.from_numpy(np.ascontiguousarray(a, dtype=np.float32)).cuda() for a in (P, Minv, C, f))
 
 
+@L.on_input_device
 def fuse_depth_maps(depths, cams, images=None, normals=None, disp_thresh=0.01, num_consistent=2, normal_thresh_deg=360.0,
                     capacity=None):
     """depths (N,H,W) fp32 cuda (0 = no measurement), cams = cameras_from_krt(...), images (N,H,W,3|4) fp32 or None,

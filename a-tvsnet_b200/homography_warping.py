@@ -10,6 +10,7 @@ from . import _lib as L
 from .flags import FLAGS
 
 
+@L.on_input_device
 def get_homographies(left_cam, right_cam, depth_num, depth_start, depth_interval):
     """(B,2,4,4) x2, int, (B,), (B,) -> (B,D,3,3) fp32.  homography_warping.py:179-227."""
     L.require_cuda(left_cam, right_cam)
@@ -33,6 +34,7 @@ def _method_code(method):
     raise ValueError("method must be 'bilinear' or 'nearest'")
 
 
+@L.on_input_device
 def homography_warping(input_image, homography, method='bilinear', output_mask=False):
     """(B,H,W,C), (B,3,3) -> (B,H,W,C) [, bool (B,H,W,1)].  homography_warping.py:230-271."""
     L.require_cuda(input_image, homography)
@@ -47,6 +49,7 @@ def homography_warping(input_image, homography, method='bilinear', output_mask=F
     return (out, mask.bool()) if output_mask else out
 
 
+@L.on_input_device
 def homography_warping_by_depth(input_image, left_cam, right_cam, depth_image, output_mask=False,
                                 method='bilinear'):
     """homography_warping.py:108-176.  depth_image (B,H,W,1)."""

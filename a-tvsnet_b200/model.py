@@ -39,6 +39,7 @@ def _prob2depth(prob_volume, depth_start, depth_interval, up, out_prob_map):
     return est, pm
 
 
+@L.on_input_device
 def prob2depth(prob_volume, depth_num, depth_start, depth_interval, out_prob_map=False):
     """(B,D,H,W) logits -> (B,H,W,1) [, prob map (B,H,W,1)].  model.py:80-109 (+ :13-65)."""
     if int(depth_num) != prob_volume.shape[1]:
@@ -47,6 +48,7 @@ def prob2depth(prob_volume, depth_num, depth_start, depth_interval, out_prob_map
     return (est, pm) if out_prob_map else est
 
 
+@L.on_input_device
 def prob2depth_upsample(prob_volume, depth_num, depth_start, depth_interval, out_prob_map=False):
     """model.py:113-129: (est, est_up[, prob, prob_up]); the x4 bilinear logit upsample
     (:68-76) is fused into the soft-argmin kernel and never materialised."""
@@ -59,11 +61,13 @@ def prob2depth_upsample(prob_volume, depth_num, depth_start, depth_interval, out
     return est, est_up
 
 
+@L.on_input_device
 def output_conv(cost_volume, reuse=AUTO_REUSE):
     """model.py:132-135: (B,D,H,W,C) -> (B,D,H,W)."""
     return OutputConv({'data': cost_volume}, is_training=True, reuse=reuse).get_output().squeeze(-1)
 
 
+@L.on_input_device
 def output_conv_refine(cost_volume, reuse=AUTO_REUSE):
     """model.py:137-140."""
     return OutputConv_refine({'data': cost_volume}, is_training=True, reuse=reuse).get_output().squeeze(-1)
@@ -72,6 +76,7 @@ def output_conv_refine(cost_volume, reuse=AUTO_REUSE):
 _MODES = {'concat': 0, 'warped_only': 1, 'l1_masked': 2}
 
 
+@L.on_input_device
 def build_cost_volume(ref_feature, view_feature, cams, depth_num, depth_start, depth_interval, ref_id, view_id,
                       output_homo=False, warp_ref=False, mode='concat', out_dtype=torch.float32):
     """model.py:157-200: (B,h,w,F) x2, cams (B,N,2,4,4) -> (B,D,h,w,2F) [, (B,D,3,3)].
@@ -105,6 +110,7 @@ def build_cost_volume(ref_feature, view_feature, cams, depth_num, depth_start, d
     return (out, hv) if output_homo else out
 
 
+@L.on_input_device
 def cost_volume_reasoning(cost_volume, output_prob=True, output_filtered_cost=False, reuse=AUTO_REUSE):
     """model.py:204-223 (CRM): (B,D,h,w,2F) -> (B,D,h,w) and/or (B,D,h,w,C) fp32."""
     if output_prob:
@@ -118,6 +124,7 @@ def cost_volume_reasoning(cost_volume, output_prob=True, output_filtered_cost=Fa
     return tower.get_output_by_name('conv_b2_6_1').float()
 
 
+@L.on_input_device
 def cost_volume_aggregation(cost_volumes, reuse=AUTO_REUSE, keepchannel=False):
     """model.py:445-456 (AAM1): (B,D,h,w,C,N-1) -> (B,D,h,w,C) | (B,D,h,w).  A list of N-1
     (B,D,h,w,C) tensors is accepted too (avoids the host-side np.stack of example.py:150)."""
@@ -126,6 +133,7 @@ def cost_volume_aggregation(cost_volumes, reuse=AUTO_REUSE, keepchannel=False):
     return AttAggregation({'data': cost_volumes}, is_training=True, reuse=reuse).get_output().squeeze(-1)
 
 
+@L.on_input_device
 def cost_volume_aggregation_refine(cost_volumes, reuse=AUTO_REUSE, keepchannel=False):
     """model.py:460-468 (AAM2)."""
     if keepchannel:
@@ -137,6 +145,7 @@ def _cost_dtype():
     return act_dtype()
 
 
+@L.on_input_device
 def TVSNet_feature_extraction(images, view_i):
     """model.py:420-425: images (B,N,H,W,3) -> FEM feature of view ``view_i`` (B,H/4,W/4,32)."""
     from . import fem
@@ -169,6 +178,7 @@ def _tvsnet_reverse(ref, view, cams, depth_num, depth_start, depth_interval, vie
     return prob2depth(prob_vol_view, depth_num, depth_start, depth_interval, out_prob_map=False)
 
 
+@L.on_input_device
 def TVSNet_base(images, cams, depth_num, depth_start, depth_interval, view_i, ref_i=0):
     """model.py:380-395: images (B,N,H,W,3), cams (B,N,2,4,4) -> (depth_b2 (B,h,w,1), prob_vol_b2 (B,D,h,w),
     filtered_cost_volume (B,D,h,w,8))."""
@@ -176,6 +186,7 @@ def TVSNet_base(images, cams, depth_num, depth_start, depth_interval, view_i, re
     return _tvsnet_base(ref, view, cams, depth_num, depth_start, depth_interval, view_i)
 
 
+@L.on_input_device
 def TVSNet_base_siamese(images, cams, depth_num, depth_start, depth_interval, view_i, ref_i=0):
     """model.py:398-417: forward volume (ref <- view_i) and the reverse one (view_i as reference) for
     ``depth_view``; -> (depth_b2, prob_vol_b2, filtered_cost_volume, depth_view)."""
@@ -185,6 +196,7 @@ def TVSNet_base_siamese(images, cams, depth_num, depth_start, depth_interval, vi
     return depth_b2, prob_vol_b2, filtered, depth_view
 
 
+@L.on_input_device
 def TVSNet(images, cams, depth_num, depth_start, depth_interval, view_i, ref_i=0):
     """model.py:346-377, the two-view network: FEM on both images, both directions of the cost volume + CRM, then the
     refinement stage on (depth_b2, depth_view) -> refined_prob_vol (B,D,h,w) = prob_vol_b2 + residual."""
@@ -201,6 +213,7 @@ def TVSNet(images, cams, depth_num, depth_start, depth_interval, view_i, ref_i=0
     return refine.fem.add(L.f32c(prob_vol_b2), prob_residual.contiguous())
 
 
+@L.on_input_device
 def TVSNet_refine(depth_b2, depth_view, prob_vol_b2, filtered_cost_volume, images, cams, depth_num, depth_start,
                   depth_interval, view_i, ref_i=0):
     """model.py:428-441 -> (refined_prob_vol (B,D,h,w), refined_cost_volume (B,D,h,w,8))."""

@@ -329,6 +329,10 @@ class Network(object):
 
     # -- execution ---------------------------------------------------------------
     def _run(self):
+        with L.input_device(self.inputs, type(self).__name__):
+            self._execute()
+
+    def _execute(self):
         nodes = self.nodes
         order = list(nodes.keys())
         pos = {n: i for i, n in enumerate(order)}

@@ -31,12 +31,14 @@ def _cost_volume(r, v, cams, depth_num, depth_start, depth_interval, rid, vid, v
     return build_cost_volume(r, v, cams, depth_num, depth_start, depth_interval, ref_id=rid, view_id=vid, out_dtype=dt)
 
 
+@L.on_input_device
 def features_act(features):
     """(B,N,h,w,F) fp32 feature maps -> the same in the 16-bit activation dtype, ONE conversion per frame for all the
     passes that warp a view (forward passes warp the sources, reverse passes the reference); None on the fp32 path."""
     return N.to_act(features) if N.act_dtype() in N.HALF_DTYPES else None
 
 
+@L.on_input_device
 def stage1_forward(features, cams, depth_num, depth_start, depth_interval, view_i, features16=None):
     """forward half of TVSNet_base_siamese (model.py:409-411): ref <- view_i.  Returns the 8-ch
     filtered volume (activation dtype) and the prob logits (fp32)."""
@@ -46,6 +48,7 @@ def stage1_forward(features, cams, depth_num, depth_start, depth_interval, view_
     return tower.get_output_by_name('conv_b2_6_1'), tower.get_output().squeeze(-1)
 
 
+@L.on_input_device
 def stage1_reverse(features, cams, depth_num, depth_start, depth_interval, view_i, features16=None, confidence=False):
     """reverse half (model.py:413-415): view_i as reference -> depth_view (B,h,w,1); with ``confidence`` the pair
     (depth_view, its probability map (B,h,w,1)), both from the same soft-argmin launch."""
@@ -56,6 +59,7 @@ def stage1_reverse(features, cams, depth_num, depth_start, depth_interval, view_
     return (depth_view, prob_map) if confidence else depth_view
 
 
+@L.on_input_device
 def stage1_view(features, cams, depth_num, depth_start, depth_interval, view_i, siamese=True):
     """TVSNet_base_siamese (model.py:398-417) keeping the 8-ch filtered volume in the activation
     dtype.  Returns (filtered (B,D,h,w,8), prob logits (B,D,h,w) fp32, depth_view | None)."""
@@ -101,6 +105,7 @@ def reduce_partials(nd, world, rank, group, finish, gather_dtype):
     return full[:V]
 
 
+@L.on_input_device
 def aggregate(filtered_views, scope='attention_aggregate', group=None, rank=0, world=1, raw=None):
     """AAM (network.py:379-408) over this rank's views; with ``group`` the softmax over views is completed across
     ranks: all-reduce(MAX) of the local logit max (as bf16: any shift that is the same on every rank is exact for the
@@ -158,6 +163,7 @@ def shard_views(n_views, rank, world):
     return [v for v in range(1, n_views) if (v - 1) % world == rank]
 
 
+@L.on_input_device
 def run_multiview(features, cams, depth_num, siamese=True, upsample=True, group=None, rank=0, world=1, confidence=False):
     """features (B,N,h,w,F) fp32, cams (B,N,2,4,4) -> dict(depth (B,h,w,1), depth_up (B,4h,4w,1),
     prob_volume_agg, cost_volume_agg, depth_views).  example.py:144-158 + :109 (x4 upsample).
@@ -237,6 +243,7 @@ def run_multiview(features, cams, depth_num, siamese=True, upsample=True, group=
     return out
 
 
+@L.on_input_device
 def run_example_schedule(images, cams, depth_num, features=None, confidence=False):
     """The whole four-stage schedule of example.py:144-181 on the device, images in:
       I   per source view: FEM features -> TVSNet_base_siamese -> (filtered cost, prob volume, depth_view)
@@ -273,6 +280,7 @@ def run_example_schedule(images, cams, depth_num, features=None, confidence=Fals
     return out
 
 
+@L.on_input_device
 def run_twoview(images, cams, depth_num, confidence=False):
     """The two-view driver of example.py:219-272 (run_test_twoview; taken when only two views exist, example.py:344-347):
     TVSNet (FEM on both images, both directions, refinement) -> prob2depth_upsample.  images (B,2,H,W,3) raw 0..255 BGR,
@@ -300,6 +308,7 @@ def inverse_to_depth(out, twoview=False):
     return 1.0 / out
 
 
+@L.on_input_device
 def run_example(images, cams, depth_num=None, confidence=False):
     """example.py:main dispatch (:344-347): the multi-view schedule for more than two views, the two-view network
     otherwise.  Returns the final x4 inverse-depth map (B,H,W,1) and ``pred`` = depth (what example.py saves); with
@@ -341,28 +350,19 @@ def load_example(data_root, view_num=5):
             np.load(gt) if os.path.exists(gt) else None)
 
 
-class FrameStream(object):
-    """Depth maps for a stream of frames that live in PINNED HOST memory (what a reader thread hands over): the step is
-    captured once as a CUDA graph over fixed device buffers, and the host->device copy of frame i+1 and the
-    device->host copy of depth map i-1 run on their own streams while frame i computes (double-buffered staging).
+class _DeviceStream(object):
+    """What FrameStream keeps on one device: the step captured as a CUDA graph over fixed device buffers, the
+    double-buffered staging of inputs and outputs, the two copy streams and the pinned host outputs."""
 
-        fs = FrameStream(feats_shape, cams_shape, depth_num, device)
-        for depth_h in fs.run(frames):      # frames: iterable of (feats_pinned, cams_pinned)
-            ...                              # depth_h: pinned (B,4h,4w,1) fp32, valid until two frames later
-
-    With ``confidence=True`` the graph also computes the x4 probability map (run_multiview's prob_map_up) and ``run``
-    yields pinned (depth_h, confidence_h) pairs of that shape, copied and kept valid like the depth map alone.
-    """
-
-    def __init__(self, feats_shape, cams_shape, depth_num, device, siamese=True, confidence=False):
-        self.device = torch.device(device)
+    def __init__(self, feats_shape, cams_shape, depth_num, device, siamese, confidence):
+        self.device = device
         self.depth_num = int(depth_num)
-        dev = self.device
-        self.feats = torch.zeros(feats_shape, dtype=torch.float32, device=dev)
-        self.cams = torch.zeros(cams_shape, dtype=torch.float32, device=dev)
-        self.stage_f = [torch.empty_like(self.feats) for _ in range(2)]
-        self.stage_c = [torch.empty_like(self.cams) for _ in range(2)]
-        self.s_in, self.s_out = torch.cuda.Stream(device=dev), torch.cuda.Stream(device=dev)
+        with torch.cuda.device(device):
+            self.feats = torch.zeros(feats_shape, dtype=torch.float32, device=device)
+            self.cams = torch.zeros(cams_shape, dtype=torch.float32, device=device)
+            self.stage_f = [torch.empty_like(self.feats) for _ in range(2)]
+            self.stage_c = [torch.empty_like(self.cams) for _ in range(2)]
+            self.s_in, self.s_out = torch.cuda.Stream(device=device), torch.cuda.Stream(device=device)
         self.siamese = siamese
         self.confidence = confidence
         self.graph = None
@@ -372,7 +372,7 @@ class FrameStream(object):
         return run_multiview(self.feats, self.cams, self.depth_num, siamese=self.siamese, confidence=self.confidence)
 
     def _capture(self):
-        for _ in range(3):      # eager warm-up: packs the weights, sets kernel attributes, fills the allocator
+        for _ in range(3):      # eager warm-up: copies and packs the weights, sets kernel attributes, fills the allocator
             self._step()
         torch.cuda.synchronize(self.device)
         s = torch.cuda.Stream(device=self.device)
@@ -383,27 +383,29 @@ class FrameStream(object):
                 res = self._step()
                 self.out = [res[k] for k in (('depth_up', 'prob_map_up') if self.confidence else ('depth_up',))]
         torch.cuda.current_stream(self.device).wait_stream(s)
-        # per output: staging slot k on the device and its pinned host copy, k = frame index & 1
+        # per output: staging slot k on the device and its pinned host copy, k = this device's frame index & 1
         self.stage_o = [[torch.empty_like(o) for o in self.out] for _ in range(2)]
         self.host_o = [[torch.empty(o.shape, dtype=torch.float32).pin_memory() for o in self.out] for _ in range(2)]
 
-    def run(self, frames):
-        """generator over pinned host depth maps, one per frame, in order (each is yielded once its copy is complete);
-        (depth, confidence) pairs with ``confidence=True``."""
-        main = torch.cuda.current_stream(self.device)
-        first = True
-        free = [None, None]          # staging slot reusable once the step that read it has copied it out
-        done = [None, None]          # D2H of slot complete
-        pending = []
-        for i, (fh, ch) in enumerate(frames):
-            k = i & 1
-            if first:
-                # the graph is captured on real data of the first frame (BN statistics of zeros would be degenerate)
+    def begin(self):
+        """start of a FrameStream.run: frames dealt to this device are counted from 0 again"""
+        self.n = 0
+        self.free = [None, None]     # staging slot reusable once the step that read it has copied it out
+        self.done = [None, None]     # D2H of slot complete
+        self.main = torch.cuda.current_stream(self.device)
+
+    def push(self, fh, ch):
+        """enqueue one frame (nothing here waits for the device once the graph exists) -> (event, pinned result),
+        the result complete once the event is"""
+        k = self.n & 1
+        self.n += 1
+        main, free, done = self.main, self.free, self.done
+        with torch.cuda.device(self.device):
+            if self.graph is None:
+                # captured on real data of the first frame dealt to this device (BN statistics of zeros are degenerate)
                 self.feats.copy_(fh, non_blocking=True)
                 self.cams.copy_(ch, non_blocking=True)
-                if self.graph is None:
-                    self._capture()
-                first = False
+                self._capture()
             with torch.cuda.stream(self.s_in):
                 if free[k] is not None:
                     self.s_in.wait_event(free[k])
@@ -418,7 +420,7 @@ class FrameStream(object):
             free[k].record(main)
             self.graph.replay()
             if done[k] is not None:
-                main.wait_event(done[k])          # stage_o[k] / host_o[k] of frame i-2 have been drained
+                main.wait_event(done[k])          # stage_o[k] / host_o[k] of this device's frame before last are drained
             for so, o in zip(self.stage_o[k], self.out):
                 so.copy_(o, non_blocking=True)
             computed = torch.cuda.Event()
@@ -429,8 +431,57 @@ class FrameStream(object):
                     ho.copy_(so, non_blocking=True)
                 done[k] = torch.cuda.Event()
                 done[k].record(self.s_out)
-            pending.append((done[k], tuple(self.host_o[k]) if self.confidence else self.host_o[k][0]))
-            if len(pending) > 1:
+        return done[k], tuple(self.host_o[k]) if self.confidence else self.host_o[k][0]
+
+
+class FrameStream(object):
+    """Depth maps for a stream of frames that live in PINNED HOST memory (what a reader thread hands over): the step is
+    captured once per device as a CUDA graph over fixed device buffers, and the host->device copy of a device's next
+    frame and the device->host copy of its previous depth map run on their own streams while the frame computes
+    (double-buffered staging).
+
+        fs = FrameStream(feats_shape, cams_shape, depth_num, device)
+        for depth_h in fs.run(frames):      # frames: iterable of (feats_pinned, cams_pinned)
+            ...                              # depth_h: pinned (B,4h,4w,1) fp32, valid until two frames later
+
+    ``device`` is one device or a sequence of K devices: frame i then runs on device i mod K, every device with its
+    own graph (captured on the first frame dealt to it), staging buffers, copy streams and weight copies, all driven
+    from the calling thread, and ``run`` still yields the results in frame order.  The pinned buffers of frame i are
+    reused by frame i + 2K, which is enqueued when the consumer asks for frame i + K: a result stays valid until two
+    frames later on one device, and a consumer may hold the last K results it received.
+
+    With ``confidence=True`` the graph also computes the x4 probability map (run_multiview's prob_map_up) and ``run``
+    yields pinned (depth_h, confidence_h) pairs of that shape, copied and kept valid like the depth map alone.
+    """
+
+    def __init__(self, feats_shape, cams_shape, depth_num, device, siamese=True, confidence=False):
+        devices = [device] if isinstance(device, (str, int, torch.device)) else list(device)
+        if not devices:
+            raise ValueError("FrameStream: no device given")
+        self.devices = []
+        for d in devices:
+            d = torch.device('cuda', d) if isinstance(d, int) else torch.device(d)
+            if d.type != 'cuda':
+                raise ValueError("FrameStream runs on CUDA devices, got %s" % d)
+            self.devices.append(torch.device('cuda', torch.cuda.current_device()) if d.index is None else d)
+        self.confidence = confidence
+        self.lanes = [_DeviceStream(feats_shape, cams_shape, depth_num, d, siamese, confidence) for d in self.devices]
+
+    @property
+    def graph(self):
+        """the captured graph of the first device (None before its first frame)"""
+        return self.lanes[0].graph
+
+    def run(self, frames):
+        """generator over pinned host depth maps, one per frame, in order (each is yielded once its copy is complete);
+        (depth, confidence) pairs with ``confidence=True``."""
+        K = len(self.lanes)
+        for lane in self.lanes:
+            lane.begin()
+        pending = []
+        for i, (fh, ch) in enumerate(frames):
+            pending.append(self.lanes[i % K].push(fh, ch))
+            if len(pending) > K:      # every device keeps a frame queued behind the one the host waits for
                 ev, buf = pending.pop(0)
                 ev.synchronize()
                 yield buf

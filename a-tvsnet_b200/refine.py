@@ -19,6 +19,7 @@ from .homography_warping import get_homographies, homography_warping_by_depth
 from .model import build_cost_volume
 
 
+@L.on_input_device
 def transform_depth(left_depth, left_cam, right_cam):
     """homography_warping.py:275-326: (B,H,W,1) -> (B,H,W,1)."""
     L.require_cuda(left_depth, left_cam, right_cam)
@@ -30,6 +31,7 @@ def transform_depth(left_depth, left_cam, right_cam):
     return out
 
 
+@L.on_input_device
 def get_visual_hull(depth_images, cams, depth_num, depth_start, depth_interval, ref_id=0, view_num=2):
     """homography_warping.py:329-387 for view_num = 2: depth_images (B,N,H,W), cams (B,*,2,4,4) -> (B,D,H,W,1).  As in
     the reference the second slot is paired with cams[:, 1] whatever view it came from."""
@@ -52,6 +54,7 @@ def get_visual_hull(depth_images, cams, depth_num, depth_start, depth_interval, 
     return out
 
 
+@L.on_input_device
 def shallow_features(image):
     """cnn_wrapper/atvsnet.py:245-251: res_block(3, 16, 3 blocks, stride 4) + 1x1 linear conv."""
     x = fem.res_block(L.f32c(image), 'global_refine_conv0_x', 16, 3, 4, 1)
@@ -77,6 +80,7 @@ class shallow_cache(object):
         return False
 
 
+@L.on_input_device
 def extract_feature_shallow(images, ref_id=0, view_id=1):
     """model.py:143-154."""
     if _SHALLOW_MEMO is None:
@@ -133,6 +137,7 @@ def _conv_bn(x, name, stride=1, transposed=False, skips=()):
     return summ if skips else plain
 
 
+@L.on_input_device
 def CostVolRefineNet(photo_group, geo_group, prob_vol, vis_hull):
     """cnn_wrapper/atvsnet.py:295-336 -> (global_refine_3dconv6_1 (B,D,H,W,8), global_refined_cost_vol (B,D,H,W,1)), fp32
     at the interface.  With FLAGS.precision = 'fp16' | 'bf16' the U-Net runs on the tensor-core kernels (input groups
@@ -163,6 +168,7 @@ def CostVolRefineNet(photo_group, geo_group, prob_vol, vis_hull):
     return N.to_dtype(c61, torch.float32), res
 
 
+@L.on_input_device
 def refinement(init_depth_images, cams, depth_num, depth_start, depth_interval, images, prob_vol, ref_id, view_id,
                view_homographies=None, num_depths=None, depth_ref_id=None, depth_view_id=None):
     """model.py:227-339: init_depth_images (B,2,h,w,1), images (B,N,H,W,3), prob_vol (B,D,h,w) ->
@@ -199,6 +205,7 @@ def refinement(init_depth_images, cams, depth_num, depth_start, depth_interval, 
     return c61, res.squeeze(-1)
 
 
+@L.on_input_device
 def TVSNet_refine(depth_b2, depth_view, prob_vol_b2, filtered_cost_volume, images, cams, depth_num, depth_start,
                   depth_interval, view_i, ref_i=0):
     """model.py:428-441 -> (refined_prob_vol (B,D,h,w), refined_cost_volume (B,D,h,w,8))."""

@@ -9,26 +9,43 @@ import numpy as np
 import torch
 
 _STORE = {}
-_PACKED = {}
+_COPIES = {}            # device index -> {name: copy of _STORE[name] on that device}
+_PACKED = {}            # device index -> {key: packed weight image derived from that device's variables}
 _GENERATION = [0]
 
 
 def load_weights(weights, device='cuda'):
-    """weights: dict name -> array (TF layouts), or a path to an .npz with those keys."""
+    """weights: dict name -> array (TF layouts), or a path to an .npz with those keys.  The store lives on ``device``;
+    a call on another device's inputs copies each variable it reads there once (get_variable).  Loading drops every
+    copy and packed image on every device."""
     if isinstance(weights, str):
         weights = dict(np.load(weights))
     _STORE.clear()
+    _COPIES.clear()
     _PACKED.clear()
     _GENERATION[0] += 1
     for k, v in weights.items():
         _STORE[k] = torch.as_tensor(np.asarray(v, dtype=np.float32)).to(device).contiguous()
 
 
+def _current_device():
+    return torch.cuda.current_device() if torch.cuda.is_initialized() else None
+
+
 def get_variable(name):
+    """the variable on the current device (the device of the call's inputs, _lib.input_device): the loaded tensor, or
+    its copy made on first use there."""
     try:
-        return _STORE[name]
+        t = _STORE[name]
     except KeyError:
         raise KeyError("variable %r not loaded (call variables.load_weights first)" % name)
+    dev = _current_device()
+    if not t.is_cuda or t.device.index == dev:
+        return t
+    copies = _COPIES.setdefault(dev, {})
+    if name not in copies:
+        copies[name] = t.to(torch.device('cuda', dev))
+    return copies[name]
 
 
 def has_variable(name):
@@ -36,7 +53,9 @@ def has_variable(name):
 
 
 def packed_cache():
-    return _PACKED
+    """the cache of images derived from the variables (packed weights, split and padded kernels) of the current
+    device."""
+    return _PACKED.setdefault(_current_device(), {})
 
 
 def generation():

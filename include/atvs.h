@@ -10,8 +10,13 @@
  * Conventions
  *   - plain pointers and sizes only; every pointer is a DEVICE pointer unless the name
  *     ends in `_host`; the caller owns every buffer, including workspaces;
- *   - all calls are asynchronous on `stream` (a cudaStream_t passed as void*) and keep no
- *     global mutable state apart from a cache of TMA descriptors keyed by (ptr, shape);
+ *   - all calls are asynchronous on `stream` (a cudaStream_t passed as void*), which must belong to the calling
+ *     thread's current device: every launch and query applies to that device;
+ *   - state: the library holds, per device (ordinals 0..63), the fp16 saturation counter, the concurrency hint of
+ *     atvs_set_concurrency, the SM count, the shared-memory attribute of each tensor-core kernel (set race-free from
+ *     any host thread) and the occupancy of each grid-stride kernel, each set up by the first call on that device
+ *     that needs it; such a call on a device beyond 63 fails with ATVS_E_UNSUP.  Per process it holds only the
+ *     launch counter and host constants (the CRC-32C table, the driver's tensor-map encoder);
  *   - return value: 0 = ok, >0 = cudaError_t / CUresult of the failing call,
  *     <0 = argument error (ATVS_E_*); atvs_last_error() returns a thread-local message;
  *   - activations are channels-last (B,D,H,W,C), exactly the reference's NDHWC layout;
@@ -53,9 +58,9 @@ unsigned    atvs_crc32c(const void* data_host, size_t n, unsigned crc);
  * non-zero count means the checkpoint's feature scale does not fit fp16 raw storage: rerun with fp32 raw outputs. */
 long long   atvs_saturation_count(int reset);
 /* Scheduling hint (no effect on results): how many independent regularisation passes the caller runs side by side on
- * its own streams - the 2*(N-1) passes of example.py:144-158 are independent.  The persistent tensor kernels launch
- * all resident CTAs when a pass has the GPU to itself (n = 1, the default) and fewer, longer CTAs when n passes share
- * the SMs.  Returns 0.                                                                                          */
+ * its own streams of the current device - the 2*(N-1) passes of example.py:144-158 are independent.  The persistent
+ * tensor kernels launch all resident CTAs when a pass has the GPU to itself (n = 1, the default) and fewer, longer
+ * CTAs when n passes share the SMs.  Each device keeps its own hint.  Returns 0.                                */
 int         atvs_set_concurrency(int n);
 
 /* ---- get_homographies ------------------------------------------- homography_warping.py:179-227

@@ -105,7 +105,7 @@ def main():
     for fs in streams.values():
         for _ in fs.run([(feats_h, cams_h)] * 3):
             pass
-    d2h = {k: sum(t.numel() * t.element_size() for t in fs.host_o[0]) for k, fs in streams.items()}
+    d2h = {k: sum(t.numel() * t.element_size() for t in fs.lanes[0].host_o[0]) for k, fs in streams.items()}
 
     def stream_arm(fs):
         def run():
